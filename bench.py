@@ -2,6 +2,7 @@
 """bench.py -- attack iterations/s of the attack-vc perturbation loop on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload e2e|fb|emb|pm|vsmask|gl]
+                    [--dump-outputs DIR]
 
 A *step* is one attack iteration (adv = x + eps*tanh(w); forward; loss; backward; Adam) over one
 batch of synthetic 80-bin mel utterances.  Default workload = BASELINE.json configs[1]: e2e_attack,
@@ -19,8 +20,13 @@ Numbers in the JSON line
             from one eagerly launched iteration, against MEASURED_PEAKS.json.
   cpu_baseline  the oracle (PyTorch CPU restatement of the reference loop, incl. its wgrad and
             per-iteration content-encoder work) on this box's host cores, bounded sample.
-`--impl reference` times that CPU loop alone (the reference is Python/PyTorch; /root/reference does
-not travel to the GPU box, the oracle is bit-identical to it -- tests/test_oracle_vs_reference.py).
+`--impl reference` times that CPU loop alone (the reference is Python/PyTorch and is not part of this
+repository; the oracle is bit-identical to it -- tests/test_oracle_vs_reference.py).
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned for its last step as
+DIR/<name>.npy (float32; rank 0).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.  Arrays are sampled along their first axis with a fixed
+seed where the files would otherwise exceed 64 MB in all.
 """
 from __future__ import annotations
 
@@ -58,6 +64,29 @@ def load_peaks():
         return {"hbm_gbs": d["hbm_gbs"], "bf16_tflops": d["bf16_tflops"], "bf16_tflops_sustained": d.get("bf16_tflops_sustained"),
                 "source": "measured (MEASURED_PEAKS.json)"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback (B200_PROFILING.md)"}
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: every tensor of `arrays` as path/<name>.npy in float32, all files together within DUMP_BYTES.
+    An array over its share keeps a fixed, seeded subset of its rows (first axis; elements when one row is too big)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())        # small arrays first: the big ones share the rest
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(items):
+        a = t.detach().float().cpu().numpy().reshape(t.shape or (1,))
+        share = left // (len(items) - i) - 4096                        # 4096: room for the .npy header
+        if a.nbytes > share:
+            if a[0].nbytes > share:
+                a = a.reshape(-1)
+            keep = np.sort(np.random.default_rng(0).choice(a.shape[0], share // a[0].nbytes, replace=False))
+            a = a[keep]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= os.path.getsize(os.path.join(path, name + ".npy"))
+        print(f"bench.py: {path}/{name}.npy {list(a.shape)} of {list(t.shape)}", file=sys.stderr)
 
 
 class ClockSampler:
@@ -287,12 +316,15 @@ def pm_arm(args, rank, world, local):
             return v
         t = torch.tensor([v], device=dev, dtype=torch.float64); dist.all_reduce(t, op=dist.ReduceOp.MAX); return float(t.item())
 
+    last = {}                                 # what the last train_step returned (--dump-outputs)
+
     def step(xs, ys):
         if vsmask:
             return trainer.step(xs, ys, lr=1e-3)
         r = eng.train_step(xs, reuse_buffers=True)
         if world > 1:
             dist.all_reduce(r["flat"])        # the gradients of the global batch: one 24.4 MB collective
+        last.update(r)
         return r["loss"]
     launches_of = lambda: eng.kernel_launches + (se.kernel_launches if se is not None else 0)      # noqa: E731
     for _ in range(W):
@@ -309,6 +341,13 @@ def pm_arm(args, rank, world, local):
     ms = mx(e0.elapsed_time(e1))
     launches = launches_of() - l0
     value = K * B * world / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        if vsmask:      # the step returns the loss; the weights and BatchNorm statistics it updated are read back
+            state = trainer.state_dict()
+            dump_outputs(args.dump_outputs, {"loss": loss, "state": torch.cat([v.reshape(-1) for v in state.values()])})
+        else:
+            dump_outputs(args.dump_outputs, {"loss": last["loss"], "out": last["out"], "grads": last["flat"],
+                                             "new_stats": torch.cat([v.reshape(-1) for v in last["new_stats"].values()])})
     # eval forward alone
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     fwd_rate = None
@@ -418,13 +457,15 @@ def gl_arm(args, rank, world, local):
     with ClockSampler(local) as clk:
         e0.record()
         for _ in range(K):
-            eng.mel2wav(mel, n_iter=100)
+            wav = eng.mel2wav(mel, n_iter=100)
         e1.record()
         torch.cuda.synchronize(dev)
         if world > 1:
             dist.barrier()
     ms = mx(e0.elapsed_time(e1))
     launches = eng.kernel_launches - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"wav": wav})
     t0 = time.perf_counter()
     for _ in range(K):
         w = eng.mel2wav(host.to(dev, non_blocking=True), n_iter=100).cpu()
@@ -485,7 +526,12 @@ def main():
     ap.add_argument("--workload", default="e2e", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the batched side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1: every rate is the timed steps over their time")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -554,6 +600,7 @@ def main():
     sess = eng.begin(kind, inp["vc_tgt"], inp["adv_tgt"], 0.1, W + K + 1, vc_src=src, w0=inp["w0"], want_loss=True)
     launches_per_iter = sess.launches_per_iter
     sess.step(W)
+    prof = sess.profile()                                   # one eager iteration, events around every launch
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     with ClockSampler(local) as clk:
@@ -564,11 +611,12 @@ def main():
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = clk.summary()
     value = K * B * world / (ms / 1e3)
-    prof = sess.profile()                                   # one eager iteration, events around every launch
-    _, info = sess.end()
+    adv, info = sess.end()                                  # the timed steps are the session's last iterations
     losses = info["losses"][: W + K + 1]
     if not bool(torch.isfinite(losses).all()):
         raise SystemExit("bench.py: non-finite loss")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"adv": adv, "losses": losses})
 
     # ---- roofline of the dominant kernel class (conv) from the per-launch event times ---------------
     peaks = load_peaks()

@@ -6,7 +6,7 @@ Functional PyTorch restatement (fp32 or fp64) of ``/root/reference/models/predic
   PredictiveModel    :53-110 7 down blocks, 5 up blocks, tanh
 Only ``tests/`` and bench legs may import it.  Pinned by executing the unmodified reference module
 (loaded by file path: ``models.py`` shadows the ``models/`` directory, SURVEY §2 #8) in
-tests/test_oracle_vs_reference.py and by the golden vectors of tests/tools/make_golden.py.
+tests/test_oracle_vs_reference.py, and on every run by tests/golden/vsmask_predictive.npz (tests/tools/make_golden.py).
 """
 from __future__ import annotations
 

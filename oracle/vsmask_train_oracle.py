@@ -14,7 +14,8 @@ placeholder, train_predictive.py:198-213), as for the universal header.
 
 Pinned by tests/test_oracle_vs_reference.py: the same step driven through the reference's own PredictiveModel module
 and the reference's own apply_weighted_constraint source (extracted from utils/audio.py: torchaudio is not installed, so
-the module itself cannot be imported) is bit-identical.  Only ``tests/`` and bench legs may import this file.
+the module itself cannot be imported) is bit-identical; on every run by tests/golden/vsmask_train.npz.  Only ``tests/``
+and bench legs may import this file.
 """
 from __future__ import annotations
 

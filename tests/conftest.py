@@ -8,7 +8,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
+# a checkout of the original attack-vc project (with the VSMask models/ and utils/), for test_oracle_vs_reference.py
+# and tests/tools/make_golden.py; it is not part of this repository
+REFERENCE = os.environ.get("ATTACK_VC_REFERENCE", "")
 
 
 def pytest_configure(config):

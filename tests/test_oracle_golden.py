@@ -39,3 +39,56 @@ def test_attack_golden(oracle, cpu_model, golden, name):
         np.testing.assert_allclose(o["adv"].numpy(), g["adv"], rtol=0, atol=2e-5)
     # perturbation bound (attack_utils.py:40): |adv - x| <= eps up to one rounding of the sum
     assert np.abs(g["adv"] - g["vc_tgt"]).max() <= 0.1 * (1 + 1e-6)
+
+
+# ---- VSMask side: the cases of test_oracle_vs_reference.py, pinned by tests/golden/vsmask_*.npz (tests/tools/make_golden.py) ----
+
+def _check_sampled(g, prefix, tensors, rtol, atol):
+    """Seeded element samples and whole-tensor norms stored by make_golden._sample_into."""
+    assert {k.split("__")[2] for k in g if k.startswith(prefix + "__norm__")} == set(tensors)
+    for name, t in tensors.items():
+        a = t.detach().double().reshape(-1).numpy()
+        np.testing.assert_allclose(a[g[f"{prefix}__idx__{name}"]], g[f"{prefix}__val__{name}"], rtol=rtol, atol=atol, err_msg=name)
+        # atol too: the gradient of a conv bias that feeds BatchNorm is zero up to rounding
+        np.testing.assert_allclose(np.linalg.norm(a), g[f"{prefix}__norm__{name}"], rtol=rtol, atol=atol, err_msg=name)
+
+
+def test_state_dict_keys_golden(cpu_model, golden):
+    from oracle.predictive_oracle import pm_make_state_dict
+    g = golden("vsmask_keys")
+    for tag, items in (("adainvc", cpu_model.state_dict().items()), ("predictive", pm_make_state_dict(0).items())):
+        assert [k for k, _ in items] == g[f"{tag}_keys"].tolist()
+        assert [",".join(map(str, v.shape)) for _, v in items] == g[f"{tag}_shapes"].tolist()
+
+
+def test_header_optimize_golden(oracle, cpu_model, golden):
+    g = golden("vsmask_header")
+    inp = oracle.make_inputs("emb", 3, 100, seed=4)
+    src, tgt = inp["vc_tgt"].unsqueeze(1) * 0.6, inp["adv_tgt"].unsqueeze(1) * 0.6
+    o = oracle.run_header(cpu_model, src, tgt, 5, epsilon=0.003)
+    # 1 vs 8 host threads move the 5-step header by up to 6e-7 (of its 3e-3 bound)
+    np.testing.assert_allclose(o["header"].numpy(), g["header"], rtol=0, atol=5e-6)
+
+
+def test_predictive_golden(golden):
+    from oracle import predictive_oracle as P
+    g = golden("vsmask_predictive")
+    sd = P.pm_make_state_dict(0)
+    x = torch.randn(3, 1, 80, 100, generator=torch.Generator().manual_seed(5))
+    t = P.pm_train_step(sd, x)
+    np.testing.assert_allclose(t["loss"].numpy(), g["loss"], rtol=1e-5)
+    _check_sampled(g, "out", {"eval": P.pm_forward(sd, x, training=False), "train": t["out"], "grad_x": t["grad_x"]}, 1e-4, 1e-7)
+    _check_sampled(g, "grad", t["grads"], 1e-4, 1e-8)
+    _check_sampled(g, "stats", t["new_stats"], 1e-5, 1e-7)
+
+
+def test_vsmask_train_golden(cpu_model, golden):
+    from oracle import predictive_oracle as P
+    from oracle import vsmask_train_oracle as V
+    g = golden("vsmask_train")
+    sd = P.pm_make_state_dict(0)
+    gen = torch.Generator().manual_seed(21)
+    batches = [(0.5 * torch.randn(3, 1, 80, 100, generator=gen), 0.5 * torch.randn(3, 1, 80, 100, generator=gen)) for _ in range(3)]
+    o = V.train_steps(sd, cpu_model.speaker_encoder, batches, lr=1e-3, future_steps=10, eps=(0.01, 0.005, 0.008), lambda_param=0.5)
+    np.testing.assert_allclose(o["losses"].numpy(), g["losses"], rtol=1e-5)
+    _check_sampled(g, "update", {k: v - sd[k] for k, v in o["state"].items() if v.dtype.is_floating_point}, 1e-3, 1e-6)

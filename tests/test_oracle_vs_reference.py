@@ -1,4 +1,9 @@
-"""Oracle == unmodified reference, executed here (build container only; skipped on the GPU box)."""
+"""Oracle == unmodified reference, bit for bit, executed here.  Runs when ATTACK_VC_REFERENCE names a checkout of the
+original project (it is not part of this repository).  Every case here is also pinned without it by tests/golden, in
+test_oracle_golden.py: the AdaIN-VC forward and attack vectors were made from the reference; the vsmask_* vectors
+(state-dict keys, header, PredictiveModel, trainer steps) were made from the oracle, which this module holds bit-identical
+to the reference on the same cases.  Each file's "source" entry says which; tests/tools/make_golden.py remakes them from
+the reference when ATTACK_VC_REFERENCE is set."""
 import os
 import sys
 
@@ -7,7 +12,8 @@ import torch
 
 from conftest import REFERENCE
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not (REFERENCE and os.path.isdir(REFERENCE)),
+                                reason="set ATTACK_VC_REFERENCE to a checkout of the original attack-vc project")
 
 
 @pytest.fixture(scope="module")
@@ -127,22 +133,15 @@ def _ref_weighted_constraint():
     return lambda p, e1, e2, e3: ns["apply_weighted_constraint"](None, p, epsilon1=e1, epsilon2=e2, epsilon3=e3)
 
 
-def test_vsmask_train_step_bit_exact(ref_model):
-    """oracle.vsmask_train_oracle.train_steps == the loop body of train_predictive.py:92-126 driven through the reference's
-    PredictiveModel module, the reference's apply_weighted_constraint and the reference's AdaIN-VC speaker encoder, with the
-    two documented repairs (crop to F mel rows, constraint on squeeze(1))."""
-    from oracle import predictive_oracle as P
-    from oracle import vsmask_train_oracle as V
+def _ref_train_steps(ref_model, sd, batches, eps):
+    """The loop body of train_predictive.py:92-126 driven through the reference's PredictiveModel module, the reference's
+    apply_weighted_constraint and the reference's AdaIN-VC speaker encoder, with the two documented repairs (crop to F
+    mel rows, constraint on squeeze(1)).  Returns the losses, the final state dict and how many elements were clamped."""
     constraint = _ref_weighted_constraint()
     pm = _ref_predictive()
-    sd = P.pm_make_state_dict(0)
     pm.load_state_dict(sd, strict=True)
-    g = torch.Generator().manual_seed(21)
-    batches = [(0.5 * torch.randn(3, 1, 80, 100, generator=g), 0.5 * torch.randn(3, 1, 80, 100, generator=g)) for _ in range(3)]
-    # eps an order of magnitude below the defaults: this synthetic model predicts |p| ~ 1e-2, and the clamp must be live
     enc = lambda m: ref_model.speaker_encoder(m.squeeze(1))
     opt = torch.optim.Adam(pm.parameters(), lr=1e-3)                       # train_predictive.py:57
-    eps = (0.01, 0.005, 0.008)
     losses = []
     pm.train()                                                             # :64
     n_clamped = 0
@@ -161,9 +160,22 @@ def test_vsmask_train_step_bit_exact(ref_model):
         loss = mse(e_p, e_t) - 0.5 * mse(e_p, e_s)                         # :119-122
         opt.zero_grad(); loss.backward(); opt.step()                       # :125-127
         losses.append(float(loss.detach()))
+    return losses, pm.state_dict(), n_clamped
+
+
+def test_vsmask_train_step_bit_exact(ref_model):
+    """oracle.vsmask_train_oracle.train_steps == the reference's training loop (_ref_train_steps)."""
+    from oracle import predictive_oracle as P
+    from oracle import vsmask_train_oracle as V
+    sd = P.pm_make_state_dict(0)
+    g = torch.Generator().manual_seed(21)
+    batches = [(0.5 * torch.randn(3, 1, 80, 100, generator=g), 0.5 * torch.randn(3, 1, 80, 100, generator=g)) for _ in range(3)]
+    # eps an order of magnitude below the defaults: this synthetic model predicts |p| ~ 1e-2, and the clamp must be live
+    eps = (0.01, 0.005, 0.008)
+    losses, state, n_clamped = _ref_train_steps(ref_model, sd, batches, eps)
     assert n_clamped > 0                                                   # the clamp (and its mask in the backward) is exercised
     o = V.train_steps(sd, ref_model.speaker_encoder, batches, lr=1e-3, future_steps=10, eps=eps, lambda_param=0.5)
     assert o["losses"].tolist() == losses
-    for k, v in pm.state_dict().items():
+    for k, v in state.items():
         if v.dtype.is_floating_point:
             assert torch.equal(v, o["state"][k]), k

@@ -1,7 +1,9 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (/root/reference) on CPU.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference on CPU.
 
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/tools/make_golden.py
+ATTACK_VC_REFERENCE names a checkout of the original attack-vc project:
+    ATTACK_VC_REFERENCE=<dir> python tests/tools/make_golden.py [case ...]
+Without it only the vsmask_* cases can be made, from the oracle instead of the reference (see vsmask_vectors):
+    python tests/tools/make_golden.py vsmask_keys vsmask_header vsmask_predictive vsmask_train
 Weights: oracle.make_state_dict(seed=0) loaded into the reference's AdaInVC with strict=True.
 Inputs:  oracle.make_inputs(...).  The reference's own attack functions draw w0 from the global
 RNG (attack_utils.py:30,68,112); we seed it, draw the same tensor first, and store it.
@@ -16,10 +18,11 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
-
-import attack_utils as RA  # noqa: E402  (reference)
-import models as RM  # noqa: E402  (reference)
+REFERENCE = os.environ.get("ATTACK_VC_REFERENCE", "")
+if REFERENCE:
+    sys.path.insert(0, REFERENCE)
+    import attack_utils as RA  # noqa: E402  (reference)
+    import models as RM  # noqa: E402  (reference)
 from oracle import adainvc_oracle as O  # noqa: E402
 
 torch.set_num_threads(8)
@@ -121,7 +124,102 @@ def model_vectors():
     print("model_fwd", emb.shape, mu.shape, out.shape)
 
 
+def _sample_into(d, prefix, tensors, k=64):
+    """Per tensor: a seeded sample of k elements (flat index + value) and the fp64 norm of the whole tensor, so that a
+    few kB pin each of the 6.09 M-element gradient / weight sets of the PredictiveModel."""
+    rng = np.random.default_rng(0)
+    for name, t in tensors.items():
+        a = t.detach().double().reshape(-1).numpy()
+        idx = np.sort(rng.choice(a.size, min(k, a.size), replace=False))
+        d[f"{prefix}__idx__{name}"] = idx.astype(np.int32)
+        d[f"{prefix}__val__{name}"] = a[idx].astype(np.float32)
+        d[f"{prefix}__norm__{name}"] = np.float64(np.linalg.norm(a))
+
+
+def vsmask_vectors(name):
+    """The cases of tests/test_oracle_vs_reference.py that the attack vectors above do not cover: state-dict keys and
+    shapes, UniversalPerturbationHeader.optimize, the PredictiveModel eval / train forward with its backward, and three
+    VSMask trainer steps.  Inputs are the same seeded ones; they are regenerated by the test, not stored.
+    With ATTACK_VC_REFERENCE the reference's own modules compute them (as test_oracle_vs_reference.py drives them);
+    without it the oracle does, which that module asserts to be bit-identical to the reference on exactly these
+    cases.  The file records which one it was ("source")."""
+    from attack_vc_b200.synthetic import pm_make_state_dict
+    from oracle import predictive_oracle as P
+    from oracle import vsmask_train_oracle as V
+    cpu_model = O.OracleAdaInVC(O.SYNTH_CONFIG, seed=0)
+    if REFERENCE:
+        sys.path.insert(0, os.path.join(ROOT, "tests"))
+        import test_oracle_vs_reference as TR
+        model = RM.AdaInVC(O.SYNTH_CONFIG)
+        model.load_state_dict(O.make_state_dict(seed=0), strict=True)
+    else:
+        model = cpu_model
+    d = {"source": np.array("reference" if REFERENCE else "oracle")}
+    sd = pm_make_state_dict(0)
+    if name == "vsmask_keys":
+        pm_keys = list(TR._ref_predictive().state_dict().items()) if REFERENCE else list(sd.items())
+        for tag, items in (("adainvc", list(model.state_dict().items())), ("predictive", pm_keys)):
+            d[f"{tag}_keys"] = np.array([k for k, _ in items])
+            d[f"{tag}_shapes"] = np.array([",".join(map(str, v.shape)) for _, v in items])
+    elif name == "vsmask_header":
+        inp = O.make_inputs("emb", 3, 100, seed=4)
+        src, tgt = inp["vc_tgt"].unsqueeze(1) * 0.6, inp["adv_tgt"].unsqueeze(1) * 0.6
+        if REFERENCE:
+            import importlib.util
+            spec = importlib.util.spec_from_file_location("ref_header_model", os.path.join(REFERENCE, "models", "header_model.py"))
+            hm = importlib.util.module_from_spec(spec)
+            spec.loader.exec_module(hm)
+            H = hm.UniversalPerturbationHeader(80, 100, device="cpu")
+            H.optimize(src, tgt, lambda m: model.speaker_encoder(m.squeeze(1)), torch.optim.Adam([H.header], lr=1e-3),
+                       num_iterations=5, epsilon=0.003, lambda_param=0.5)
+            header = H.header.detach()
+        else:
+            header = O.run_header(cpu_model, src, tgt, 5, epsilon=0.003)["header"]
+        d["header"] = header.numpy()
+    elif name == "vsmask_predictive":
+        x = torch.randn(3, 1, 80, 100, generator=torch.Generator().manual_seed(5))
+        if REFERENCE:
+            pm = TR._ref_predictive()
+            pm.load_state_dict(sd, strict=True)
+            pm.eval()
+            with torch.no_grad():
+                out_eval = pm(x)
+            pm.train()
+            xin = x.clone().requires_grad_(True)
+            out = pm(xin)
+            loss = out.square().mean()
+            loss.backward()
+            grads = {n: p.grad for n, p in pm.named_parameters()}
+            grad_x = xin.grad
+            stats = {k: v for k, v in pm.state_dict().items() if "running" in k}
+        else:
+            out_eval = P.pm_forward(sd, x, training=False)
+            t = P.pm_train_step(sd, x)
+            out, loss, grads, grad_x, stats = t["out"], t["loss"], t["grads"], t["grad_x"], t["new_stats"]
+        d["loss"] = loss.detach().numpy()
+        _sample_into(d, "out", {"eval": out_eval, "train": out, "grad_x": grad_x}, k=2048)
+        _sample_into(d, "grad", grads)
+        _sample_into(d, "stats", stats, k=512)
+    elif name == "vsmask_train":
+        g = torch.Generator().manual_seed(21)
+        batches = [(0.5 * torch.randn(3, 1, 80, 100, generator=g), 0.5 * torch.randn(3, 1, 80, 100, generator=g)) for _ in range(3)]
+        eps = (0.01, 0.005, 0.008)
+        if REFERENCE:
+            losses, state, _ = TR._ref_train_steps(model, sd, batches, eps)
+        else:
+            o = V.train_steps(sd, model.speaker_encoder, batches, lr=1e-3, future_steps=10, eps=eps, lambda_param=0.5)
+            losses, state = o["losses"].tolist(), o["state"]
+        d["losses"] = np.array(losses, dtype=np.float64)
+        _sample_into(d, "update", {k: v - sd[k] for k, v in state.items() if v.dtype.is_floating_point})
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **d)
+    print(name, "source", d["source"], "arrays", len(d))
+
+
 CASES = {
+    "vsmask_keys": lambda: vsmask_vectors("vsmask_keys"),
+    "vsmask_header": lambda: vsmask_vectors("vsmask_header"),
+    "vsmask_predictive": lambda: vsmask_vectors("vsmask_predictive"),
+    "vsmask_train": lambda: vsmask_vectors("vsmask_train"),
     "emb_T128_it100": lambda: case("emb_T128_it100", "emb", 1, 128, 100, (0, 1, 10, 99)),                      # BASELINE config 1
     "e2e_T64_it20": lambda: case("e2e_T64_it20", "e2e", 1, 64, 20, (0, 1, 19)),
     "fb_T64_it20": lambda: case("fb_T64_it20", "fb", 1, 64, 20, (0, 1, 19)),
