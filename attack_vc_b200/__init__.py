@@ -5,5 +5,6 @@ host-side mirror of the reference's attack interface (``engine.Engine``; the dro
 top-level ``attack_utils.py``).  Importing this package never falls back to PyTorch math: if
 ``libavc_b200.so`` is missing, using it raises."""
 from .engine import AvcError, Engine, engine_for, invalidate_engine  # noqa: F401
+from .defend import Defender  # noqa: F401,E402
 
-__all__ = ["Engine", "AvcError", "engine_for", "invalidate_engine"]
+__all__ = ["Engine", "AvcError", "engine_for", "invalidate_engine", "Defender"]

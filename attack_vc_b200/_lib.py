@@ -100,6 +100,7 @@ EXPORTS = [
     "avc_pm_trainer_end", "avc_pm_export_weights",
     "avc_audio_create", "avc_audio_destroy", "avc_audio_last_error", "avc_audio_frames", "avc_audio_samples",
     "avc_audio_wav2mel", "avc_audio_mel2wav", "avc_audio_wav2mel_batch", "avc_audio_mel2wav_batch", "avc_audio_kernel_launches",
+    "avc_audio_wav2mel_varlen", "avc_audio_mel2wav_varlen",
 ]
 
 _lib = None
@@ -196,6 +197,8 @@ def load() -> C.CDLL:
     lib.avc_audio_mel2wav.argtypes = [vp, vp, i32, i32, vp, vp]
     lib.avc_audio_wav2mel_batch.argtypes = [vp, vp, i32, i64, vp, vp]
     lib.avc_audio_mel2wav_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp]
+    lib.avc_audio_wav2mel_varlen.argtypes = [vp, vp, P(i64), i32, vp, vp, vp, vp]
+    lib.avc_audio_mel2wav_varlen.argtypes = [vp, vp, P(i32), i32, i32, vp, vp, vp, vp]
     lib.avc_audio_kernel_launches.argtypes = [vp]
     lib.avc_audio_kernel_launches.restype = i64
     lib.avc_version.argtypes = []

@@ -102,6 +102,60 @@ class AudioEngine:
             self._check(self._lib.avc_audio_mel2wav_batch(self._h, mel.data_ptr(), B, F, int(n_iter), wav.data_ptr(), st))
         return wav if batched else wav[0]
 
+    def _norm_args(self, mean: Optional[Tensor], std: Optional[Tensor]) -> Tuple[Optional[int], Optional[int], tuple]:
+        """Device pointers of the speaker-normalisation statistics (both or neither), plus the tensors to keep alive."""
+        if (mean is None) != (std is None):
+            raise ValueError("mean and std must be given together")
+        if mean is None:
+            return None, None, ()
+        mean, std = self._vec(mean, "mean", 1), self._vec(std, "std", 1)
+        if mean.numel() != self.n_mels or std.numel() != self.n_mels:
+            raise ValueError(f"mean and std must have {self.n_mels} entries (got {mean.numel()}, {std.numel()})")
+        return mean.data_ptr(), std.data_ptr(), (mean, std)
+
+    def wav2mel_varlen(self, wavs: Sequence[Tensor], mean: Optional[Tensor] = None, std: Optional[Tensor] = None) -> List[Tensor]:
+        """file2mel over utterances of ANY lengths in ONE call (avc_audio_wav2mel_varlen): the frames of all utterances are the
+        rows of one GEMM.  With ``mean`` / ``std`` ([n_mels]) the mels come out speaker-normalised, ``(mel - mean) / std``
+        (data_utils.py:35-40).  Returns [n_frames_u, n_mels] views of one buffer, in input order."""
+        if len(wavs) == 0:
+            return []
+        flat = [self._vec(w, "wav", 1) for w in wavs]
+        ns = [int(w.numel()) for w in flat]
+        frames = [int(self._lib.avc_audio_frames(self._h, n)) for n in ns]
+        m, s, keep = self._norm_args(mean, std)
+        with torch.cuda.device(self.device):
+            wav = torch.cat(flat) if len(flat) > 1 else flat[0]
+            mel = torch.empty(max(sum(max(f, 0) for f in frames), 1), self.n_mels, device=self.device, dtype=torch.float32)
+            st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+            n_host = (C.c_int64 * len(ns))(*ns)
+            self._check(self._lib.avc_audio_wav2mel_varlen(self._h, wav.data_ptr(), n_host, len(ns), m, s, mel.data_ptr(), st))
+        del keep
+        return list(mel.split(frames))
+
+    def mel2wav_varlen(self, mels: Sequence[Tensor], n_iter: int = 100, mean: Optional[Tensor] = None,
+                       std: Optional[Tensor] = None) -> List[Tensor]:
+        """mel2wav over mels of ANY frame counts in ONE call (avc_audio_mel2wav_varlen; one Griffin-Lim loop for all of them).
+        With ``mean`` / ``std`` the inputs are speaker-normalised mels, denormalised first (``x * std + mean``,
+        data_utils.py:43-47).  Returns [hop_length * (n_frames_u - 1)] views of one buffer, in input order."""
+        if len(mels) == 0:
+            return []
+        flat = [self._vec(x, "mel", 2) for x in mels]
+        for x in flat:
+            if x.shape[-1] != self.n_mels:
+                raise ValueError(f"mel must have {self.n_mels} bins (got {x.shape[-1]})")
+        frames = [int(x.shape[0]) for x in flat]
+        ns = [int(self._lib.avc_audio_samples(self._h, f)) for f in frames]
+        m, s, keep = self._norm_args(mean, std)
+        with torch.cuda.device(self.device):
+            mel = torch.cat(flat) if len(flat) > 1 else flat[0]
+            wav = torch.empty(max(sum(max(n, 0) for n in ns), 1), device=self.device, dtype=torch.float32)
+            st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+            f_host = (C.c_int32 * len(frames))(*frames)
+            self._check(self._lib.avc_audio_mel2wav_varlen(self._h, mel.data_ptr(), f_host, len(frames), int(n_iter), m, s,
+                                                           wav.data_ptr(), st))
+        del keep
+        return list(wav.split(ns))
+
     def wav2mel_list(self, wavs: Sequence[Tensor]) -> List[Tensor]:
         """file2mel over utterances of ANY lengths (the reference loops over files, data_utils.py:65-117): equal-length
         waveforms are batched into one call each, results come back in input order."""

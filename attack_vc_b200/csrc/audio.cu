@@ -46,6 +46,15 @@ __global__ void au_preemph_kernel(const float* __restrict__ x, float* __restrict
 }
 
 // frame f, sample j = wav[reflect(f hop + j - n_fft/2)] * window[j], split into 3xTF32 planes      (librosa.stft, center=True)
+// (wav: one utterance of n samples)
+__device__ __forceinline__ void au_frame_elem(const float* __restrict__ wav, long long n, const float* __restrict__ window, float* __restrict__ hi,
+                                              float* __restrict__ lo, long long i, int f, int j, int n_fft, int hop) {
+  const float w = window[j];
+  const float v = w != 0.f ? wav[au_reflect((long long)f * hop + j - n_fft / 2, n)] * w : 0.f;
+  const float h = tf32_hi(v);
+  hi[i] = h; lo[i] = v - h;
+}
+
 // n_frames per utterance; rows of the frame matrix are (utterance, frame)
 __global__ void au_frame_kernel(const float* __restrict__ wav, long long n, const float* __restrict__ window, float* __restrict__ hi,
                                 float* __restrict__ lo, int n_frames, int B, int n_fft, int hop) {
@@ -54,10 +63,39 @@ __global__ void au_frame_kernel(const float* __restrict__ wav, long long n, cons
     const int j = (int)(i % n_fft);
     const long long r = i / n_fft;
     const int f = (int)(r % n_frames), b = (int)(r / n_frames);
-    const float w = window[j];
-    const float v = w != 0.f ? wav[(long long)b * n + au_reflect((long long)f * hop + j - n_fft / 2, n)] * w : 0.f;
-    const float h = tf32_hi(v);
-    hi[i] = h; lo[i] = v - h;
+    au_frame_elem(wav + (long long)b * n, n, window, hi, lo, i, f, j, n_fft, hop);
+  }
+}
+
+// Ragged batches (avc_audio_*_varlen): utterance u owns samples [s_off[u], s_off[u+1]) and frame rows [f_off[u], f_off[u+1]);
+// fu[r] is the utterance of frame row r.  Utterances are never empty, so the offsets are strictly increasing.
+// largest u in [0, B) with off[u] <= i
+__device__ __forceinline__ int au_find(const long long* __restrict__ off, int B, long long i) {
+  int lo = 0, hi = B - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (off[mid] <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// the pre-emphasis of au_preemph_kernel over utterances of their own lengths
+__global__ void au_preemph_varlen_kernel(const float* __restrict__ x, float* __restrict__ y, const long long* __restrict__ s_off, int B, float a) {
+  const long long tot = s_off[B];
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < tot; i += (long long)gridDim.x * blockDim.x)
+    y[i] = (i - s_off[au_find(s_off, B, i)]) ? x[i] - a * x[i - 1] : x[i];
+}
+
+__global__ void au_frame_varlen_kernel(const float* __restrict__ wav, const long long* __restrict__ s_off, const int* __restrict__ f_off,
+                                       const int* __restrict__ fu, const float* __restrict__ window, float* __restrict__ hi,
+                                       float* __restrict__ lo, long long R, int n_fft, int hop) {
+  const long long tot = R * n_fft;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < tot; i += (long long)gridDim.x * blockDim.x) {
+    const int j = (int)(i % n_fft);
+    const long long r = i / n_fft;
+    const int u = fu[r];
+    const long long s0 = s_off[u];
+    au_frame_elem(wav + s0, s_off[u + 1] - s0, window, hi, lo, i, (int)(r - f_off[u]), j, n_fft, hop);
   }
 }
 
@@ -73,8 +111,10 @@ __global__ void au_mag_kernel(const float* __restrict__ spec, float* __restrict_
 
 // mel[f][m] = clip((20 log10(max(1e-5, sum_k basis[m][k] mag[f][k])) - ref_db + max_db) / max_db, 1e-8, 1)      (:108-114)
 // one warp per output; lanes stride over the bins (fixed-order tree)
+// mean / std non-null: the speaker normalisation of data_utils.py:35-40 follows, (mel - mean[m]) / std[m], correctly rounded and
+// unfused like the numpy code
 __global__ void au_mel_kernel(const float* __restrict__ mag, const float* __restrict__ basis, float* __restrict__ mel, int n_frames, int nbin,
-                              int n_mels, float ref_db, float max_db) {
+                              int n_mels, float ref_db, float max_db, const float* __restrict__ mean, const float* __restrict__ std) {
   const long long o = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (o >= (long long)n_frames * n_mels) return;
   const int m = (int)(o % n_mels), f = (int)(o / n_mels);
@@ -84,17 +124,21 @@ __global__ void au_mel_kernel(const float* __restrict__ mag, const float* __rest
   for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
   if ((threadIdx.x & 31) == 0) {
     const float db = 20.f * log10f(fmaxf(1e-5f, s));
-    mel[o] = fminf(fmaxf((db - ref_db + max_db) / max_db, 1e-8f), 1.f);
+    const float v = fminf(fmaxf((db - ref_db + max_db) / max_db, 1e-8f), 1.f);
+    mel[o] = mean ? __fdiv_rn(__fsub_rn(v, mean[m]), std[m]) : v;
   }
 }
 
 // mag[f][k] = sum_m inv[k][m] * 10^(0.05 ((clip(mel[f][m], 0, 1) * max_db) - max_db + ref_db))                 (:151-156)
+// mean / std non-null: the input is first denormalised, x * std[m] + mean[m] (data_utils.py:43-47), correctly rounded and unfused
 __global__ void au_invmel_kernel(const float* __restrict__ mel, const float* __restrict__ inv, float* __restrict__ mag, int n_frames, int nbin,
-                                 int n_mels, float ref_db, float max_db) {
+                                 int n_mels, float ref_db, float max_db, const float* __restrict__ mean, const float* __restrict__ std) {
   extern __shared__ float au_lin[];      // [n_mels] linear-scale mel of this frame
   const int f = blockIdx.x;
   for (int m = threadIdx.x; m < n_mels; m += blockDim.x) {
-    const float v = fminf(fmaxf(mel[(long long)f * n_mels + m], 0.f), 1.f) * max_db - max_db + ref_db;
+    float x = mel[(long long)f * n_mels + m];
+    if (mean) x = __fadd_rn(__fmul_rn(x, std[m]), mean[m]);
+    const float v = fminf(fmaxf(x, 0.f), 1.f) * max_db - max_db + ref_db;
     au_lin[m] = powf(10.f, v * 0.05f);
   }
   __syncthreads();
@@ -129,25 +173,38 @@ __global__ void au_phase_kernel(const float* __restrict__ mag, const float* __re
 
 // librosa.istft after the inverse transform: y[p] = sum_f tf[f][p - f hop] w[p - f hop] / sum_f w[p - f hop]^2 (where > tiny), the
 // n_fft/2 centre padding removed.  Gather form: every output sample walks the <= ceil(n_fft / hop) frames that cover it, in order.
+// output sample s of one utterance whose n_frames time frames start at tf
+__device__ __forceinline__ float au_ola_sample(const float* __restrict__ tf, const float* __restrict__ window, long long s, int n_frames,
+                                               int n_fft, int hop) {
+  const long long p = s + n_fft / 2;
+  long long f_hi = p / hop;
+  if (f_hi > n_frames - 1) f_hi = n_frames - 1;
+  long long f_lo = (p - n_fft + hop) / hop;       // smallest f with p - f hop < n_fft  (ceil((p - n_fft + 1) / hop))
+  if (p - n_fft + 1 <= 0) f_lo = 0;
+  else f_lo = (p - n_fft + 1 + hop - 1) / hop;
+  float acc = 0.f, wss = 0.f;
+  for (long long f = f_lo; f <= f_hi; ++f) {
+    const int j = (int)(p - f * hop);
+    const float w = window[j];
+    acc = fmaf(tf[f * n_fft + j], w, acc);
+    wss = fmaf(w, w, wss);
+  }
+  return wss > 1.17549435e-38f ? acc / wss : acc;
+}
+
 __global__ void au_ola_kernel(const float* __restrict__ tf_all, const float* __restrict__ window, float* __restrict__ wav, long long n_out, int n_frames,
                               int B, int n_fft, int hop) {
-  for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n_out * B; q += (long long)gridDim.x * blockDim.x) {
-    const long long s = q % n_out;
-    const float* tf = tf_all + (q / n_out) * (long long)n_frames * n_fft;
-    const long long p = s + n_fft / 2;
-    long long f_hi = p / hop;
-    if (f_hi > n_frames - 1) f_hi = n_frames - 1;
-    long long f_lo = (p - n_fft + hop) / hop;       // smallest f with p - f hop < n_fft  (ceil((p - n_fft + 1) / hop))
-    if (p - n_fft + 1 <= 0) f_lo = 0;
-    else f_lo = (p - n_fft + 1 + hop - 1) / hop;
-    float acc = 0.f, wss = 0.f;
-    for (long long f = f_lo; f <= f_hi; ++f) {
-      const int j = (int)(p - f * hop);
-      const float w = window[j];
-      acc = fmaf(tf[f * n_fft + j], w, acc);
-      wss = fmaf(w, w, wss);
-    }
-    wav[q] = wss > 1.17549435e-38f ? acc / wss : acc;
+  for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n_out * B; q += (long long)gridDim.x * blockDim.x)
+    wav[q] = au_ola_sample(tf_all + (q / n_out) * (long long)n_frames * n_fft, window, q % n_out, n_frames, n_fft, hop);
+}
+
+// ragged: utterance u writes samples [o_off[u], o_off[u+1]) from its frame rows [f_off[u], f_off[u+1])
+__global__ void au_ola_varlen_kernel(const float* __restrict__ tf_all, const float* __restrict__ window, float* __restrict__ wav,
+                                     const long long* __restrict__ o_off, const int* __restrict__ f_off, int B, int n_fft, int hop) {
+  const long long tot = o_off[B];
+  for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < tot; q += (long long)gridDim.x * blockDim.x) {
+    const int u = au_find(o_off, B, q);
+    wav[q] = au_ola_sample(tf_all + (long long)f_off[u] * n_fft, window, q - o_off[u], f_off[u + 1] - f_off[u], n_fft, hop);
   }
 }
 
@@ -157,6 +214,15 @@ __global__ void au_deemph_kernel(float* x_all, long long n, int B, float a) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   float* x = x_all + (long long)b * n;
+  float acc = 0.f;
+  for (long long i = 0; i < n; ++i) { acc = fmaf(a, acc, x[i]); x[i] = acc; }
+}
+
+__global__ void au_deemph_varlen_kernel(float* x_all, const long long* __restrict__ o_off, int B, float a) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  float* x = x_all + o_off[b];
+  const long long n = o_off[b + 1] - o_off[b];
   float acc = 0.f;
   for (long long i = 0; i < n; ++i) { acc = fmaf(a, acc, x[i]); x[i] = acc; }
 }
@@ -367,7 +433,8 @@ int avc_audio_wav2mel_batch(avc_audio_handle* h, const float* wav, int32_t B, in
     au_mag_kernel<<<au_grid((long long)R * h->nbin, h->sm_count), 256, 0, st>>>(spec, mag, R, h->nbin, h->NP);
     CK(cudaGetLastError());
     const long long outs = (long long)R * h->d.n_mels;
-    au_mel_kernel<<<(unsigned)((outs * 32 + 255) / 256), 256, 0, st>>>(mag, h->basis, mel, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db);
+    au_mel_kernel<<<(unsigned)((outs * 32 + 255) / 256), 256, 0, st>>>(mag, h->basis, mel, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db,
+                                                                      nullptr, nullptr);
     CK(cudaGetLastError());
     h->launches += 3;
     CK(cudaStreamSynchronize(st));
@@ -385,7 +452,8 @@ int avc_audio_mel2wav_batch(avc_audio_handle* h, const float* mel, int32_t B, in
     cudaStream_t st = (cudaStream_t)stream;
     Arena mem(&h->pool, st);
     float* mag = mem.f((size_t)R * h->nbin);
-    au_invmel_kernel<<<R, 256, h->d.n_mels * sizeof(float), st>>>(mel, h->inv, mag, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db);
+    au_invmel_kernel<<<R, 256, h->d.n_mels * sizeof(float), st>>>(mel, h->inv, mag, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db,
+                                                                nullptr, nullptr);
     CK(cudaGetLastError());
     float* xh = mem.f((size_t)R * h->NP); float* xl = mem.f((size_t)R * h->NP);
     float* tf = mem.f((size_t)R * N);
@@ -406,6 +474,144 @@ int avc_audio_mel2wav_batch(avc_audio_handle* h, const float* mel, int32_t B, in
     }
     au_istft(h, mem, xh, xl, F, B, tf, wav, st);                                            // :188-189
     au_deemph_kernel<<<(B + 31) / 32, 32, 0, st>>>(wav, n_out, B, h->d.preemph);            // :162
+    CK(cudaGetLastError());
+    h->launches++;
+    CK(cudaStreamSynchronize(st));
+  });
+}
+
+}  // extern "C"
+
+namespace {
+
+template <class T>
+T* au_upload(Arena& mem, const std::vector<T>& v, cudaStream_t st) {
+  T* p = mem.raw<T>(v.size());
+  CK(cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+  return p;
+}
+
+// Offset table of a ragged batch on the device: sample offsets (B + 1), frame offsets (B + 1) and the utterance of every frame row
+struct AuTable {
+  long long* s_off = nullptr;
+  int* f_off = nullptr;
+  int* fu = nullptr;
+};
+
+AuTable au_table(Arena& mem, const std::vector<long long>& s_off, const std::vector<int>& f_off, cudaStream_t st) {
+  const int B = (int)s_off.size() - 1;
+  std::vector<int> fi(f_off);                      // [f_off (B + 1) | fu (R)]: one upload
+  fi.reserve(fi.size() + f_off[B]);
+  for (int u = 0; u < B; ++u) fi.insert(fi.end(), (size_t)(f_off[u + 1] - f_off[u]), u);
+  AuTable t;
+  t.s_off = au_upload(mem, s_off, st);
+  t.f_off = au_upload(mem, fi, st);
+  t.fu = t.f_off + B + 1;
+  return t;
+}
+
+void au_check_norm(const float* mean, const float* std) {
+  if ((mean == nullptr) != (std == nullptr)) fail(AVC_ERR_INVALID, "mean and std must both be given or both be NULL");
+}
+
+}  // namespace
+
+extern "C" {
+
+int avc_audio_wav2mel_varlen(avc_audio_handle* h, const float* wav, const int64_t* n_host, int32_t B, const float* mean, const float* std,
+                             float* mel, void* stream) {
+  if (!h) return AVC_ERR_INVALID;
+  return au_guarded(h, [&] {
+    if (!wav || !mel || !n_host || B < 1) fail(AVC_ERR_INVALID, "null tensor argument / bad batch");
+    au_check_norm(mean, std);
+    const int hop = h->d.hop_length;
+    std::vector<long long> s_off(B + 1, 0);
+    std::vector<int> f_off(B + 1, 0);
+    for (int u = 0; u < B; ++u) {
+      const long long n = n_host[u];
+      if (n <= h->d.n_fft / 2)
+        fail(AVC_ERR_INVALID, "utterance %d: waveform of %lld samples is too short for reflect padding by n_fft / 2 = %d", u, n, h->d.n_fft / 2);
+      if ((long long)f_off[u] + 1 + n / hop > (1ll << 30)) fail(AVC_ERR_INVALID, "too many frames in one call");
+      s_off[u + 1] = s_off[u] + n;
+      f_off[u + 1] = f_off[u] + 1 + (int)(n / hop);
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena mem(&h->pool, st);
+    const AuTable t = au_table(mem, s_off, f_off, st);
+    const long long S = s_off[B];
+    const int R = f_off[B], n_fft = h->d.n_fft;
+    float* pre = mem.f((size_t)S);
+    au_preemph_varlen_kernel<<<au_grid(S, h->sm_count), 256, 0, st>>>(wav, pre, t.s_off, B, h->d.preemph);
+    CK(cudaGetLastError());
+    float* fh = mem.f((size_t)R * n_fft); float* fl = mem.f((size_t)R * n_fft);
+    au_frame_varlen_kernel<<<au_grid((long long)R * n_fft, h->sm_count), 256, 0, st>>>(pre, t.s_off, t.f_off, t.fu, h->window, fh, fl, R, n_fft, hop);
+    CK(cudaGetLastError());
+    float* spec = mem.f((size_t)R * h->NP);
+    au_gemm(h, fh, fl, R, n_fft, h->wf_h, h->wf_l, h->NP, spec, st);
+    float* mag = mem.f((size_t)R * h->nbin);
+    au_mag_kernel<<<au_grid((long long)R * h->nbin, h->sm_count), 256, 0, st>>>(spec, mag, R, h->nbin, h->NP);
+    CK(cudaGetLastError());
+    const long long outs = (long long)R * h->d.n_mels;
+    au_mel_kernel<<<(unsigned)((outs * 32 + 255) / 256), 256, 0, st>>>(mag, h->basis, mel, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db,
+                                                                      mean, std);
+    CK(cudaGetLastError());
+    h->launches += 4;
+    CK(cudaStreamSynchronize(st));
+  });
+}
+
+int avc_audio_mel2wav_varlen(avc_audio_handle* h, const float* mel, const int32_t* frames_host, int32_t B, int32_t n_iter, const float* mean,
+                             const float* std, float* wav, void* stream) {
+  if (!h) return AVC_ERR_INVALID;
+  return au_guarded(h, [&] {
+    if (!mel || !wav || !frames_host || B < 1) fail(AVC_ERR_INVALID, "null tensor argument / bad batch");
+    if (n_iter < 0) fail(AVC_ERR_INVALID, "bad n_iter");
+    au_check_norm(mean, std);
+    const int N = h->d.n_fft, hop = h->d.hop_length;
+    std::vector<long long> o_off(B + 1, 0);
+    std::vector<int> f_off(B + 1, 0);
+    for (int u = 0; u < B; ++u) {
+      const int F = frames_host[u];
+      if (F < 2) fail(AVC_ERR_INVALID, "utterance %d: bad n_frames %d", u, F);
+      const long long n_out = (long long)hop * (F - 1);
+      if (n_out <= N / 2) fail(AVC_ERR_INVALID, "utterance %d: %d frames give %lld samples: too short for the STFT inside Griffin-Lim", u, F, n_out);
+      if ((long long)f_off[u] + F > (1ll << 30)) fail(AVC_ERR_INVALID, "too many frames in one call");
+      o_off[u + 1] = o_off[u] + n_out;
+      f_off[u + 1] = f_off[u] + F;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena mem(&h->pool, st);
+    const AuTable t = au_table(mem, o_off, f_off, st);
+    const int R = f_off[B];
+    float* mag = mem.f((size_t)R * h->nbin);
+    au_invmel_kernel<<<R, 256, h->d.n_mels * sizeof(float), st>>>(mel, h->inv, mag, R, h->nbin, h->d.n_mels, h->d.ref_db, h->d.max_db, mean, std);
+    CK(cudaGetLastError());
+    float* xh = mem.f((size_t)R * h->NP); float* xl = mem.f((size_t)R * h->NP);
+    float* tf = mem.f((size_t)R * N);
+    float* est = mem.f((size_t)R * h->NP);
+    float* fh = mem.f((size_t)R * N); float* fl = mem.f((size_t)R * N);
+    const unsigned gp = au_grid((long long)R * h->NP, h->sm_count);
+    const unsigned go = au_grid(o_off[B], h->sm_count), gf = au_grid((long long)R * N, h->sm_count);
+    au_phase_kernel<<<gp, 256, 0, st>>>(mag, nullptr, xh, xl, R, h->nbin, h->NP);          // X_best = spect
+    CK(cudaGetLastError());
+    h->launches += 2;
+    auto istft = [&] {
+      au_gemm(h, xh, xl, R, h->NP, h->wi_h, h->wi_l, N, tf, st);
+      au_ola_varlen_kernel<<<go, 256, 0, st>>>(tf, h->window, wav, t.s_off, t.f_off, B, N, hop);
+      CK(cudaGetLastError());
+      h->launches++;
+    };
+    for (int it = 0; it < n_iter; ++it) {                                                   // data_utils.py:183-187
+      istft();
+      au_frame_varlen_kernel<<<gf, 256, 0, st>>>(wav, t.s_off, t.f_off, t.fu, h->window, fh, fl, R, N, hop);
+      CK(cudaGetLastError());
+      au_gemm(h, fh, fl, R, N, h->wf_h, h->wf_l, h->NP, est, st);
+      au_phase_kernel<<<gp, 256, 0, st>>>(mag, est, xh, xl, R, h->nbin, h->NP);
+      CK(cudaGetLastError());
+      h->launches += 2;
+    }
+    istft();                                                                                // :188-189
+    au_deemph_varlen_kernel<<<(B + 31) / 32, 32, 0, st>>>(wav, t.s_off, B, h->d.preemph);   // :162
     CK(cudaGetLastError());
     h->launches++;
     CK(cudaStreamSynchronize(st));

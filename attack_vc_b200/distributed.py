@@ -10,7 +10,7 @@ tests of this host logic).
 """
 from __future__ import annotations
 
-from typing import Callable, Dict, Optional, Tuple
+from typing import Callable, Dict, List, Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
@@ -116,3 +116,45 @@ def sharded_header_optimize(engine, source_mel: Tensor, target_mel: Tensor, num_
     if world > 1:
         dist.all_reduce(losses, op=dist.ReduceOp.SUM, group=group)
     return header, losses
+
+
+def sharded_defend(defender, vc_tgt: Sequence[Tensor], adv_tgt: Tensor, group=None, **kw) -> List[Tensor]:
+    """``defender.defend(vc_tgt, adv_tgt, **kw)`` with the utterances split into contiguous slices, one per rank
+    (``shard_bounds``).  No collective runs during the work: given the per-utterance normaliser ``Defender`` uses, the
+    utterances are independent.  At the end ONE gather of the variable-length waveforms (lengths, then a padded
+    all-gather; NCCL on GPUs) returns every defended waveform, in input order, on every rank.  Each rank draws the
+    initial noise of its slice from its own RNG."""
+    if kw.get("return_mels"):
+        raise ValueError("sharded_defend gathers waveforms only (return_mels is not supported)")
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    B = len(vc_tgt)
+    lo, hi = shard_bounds(B, world, rank)
+    local = list(defender.defend(list(vc_tgt[lo:hi]), adv_tgt, **kw)) if hi > lo else []
+    return gather_varlen(local, B, defender.device, group=group)
+
+
+def gather_varlen(local: Sequence[Tensor], B_total: int, device, group=None) -> List[Tensor]:
+    """All-gather of 1-D tensors of different lengths, rank r holding items ``shard_bounds(B_total, world, r)``: one
+    all-gather of the lengths, one of equal-sized padded slots."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    if world == 1:
+        return list(local)
+    cap = max(-(-B_total // world), 1)
+    lens = torch.zeros(cap, dtype=torch.int64, device=device)
+    if local:
+        lens[: len(local)] = torch.tensor([int(w.numel()) for w in local], dtype=torch.int64)
+    all_lens = torch.empty(world * cap, dtype=torch.int64, device=device)
+    dist.all_gather(list(all_lens.chunk(world)), lens, group=group)
+    L = max(int(all_lens.max()), 1)
+    slot = torch.zeros(cap, L, dtype=torch.float32, device=device)
+    for k, w in enumerate(local):
+        slot[k, : w.numel()] = w
+    full = torch.empty(world * cap, L, dtype=torch.float32, device=device)
+    dist.all_gather(list(full.chunk(world)), slot, group=group)
+    n = all_lens.tolist()
+    out = []
+    for r in range(world):
+        a, b = shard_bounds(B_total, world, r)
+        out.extend(full[r * cap + k, : n[r * cap + k]] for k in range(b - a))
+    return out

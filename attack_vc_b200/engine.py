@@ -190,6 +190,24 @@ class Engine:
     def launches_per_iter(self) -> int:
         return int(self._lib.avc_launches_per_iter(self._h))
 
+    def decoder_frames(self, T_src: int) -> int:
+        """Frames of the converted utterance for a source of ``T_src`` frames (avc_decoder_frames)."""
+        return int(self._lib.avc_decoder_frames(self._h, int(T_src)))
+
+    def min_frames(self, which: str = "speaker") -> int:
+        """Shortest utterance the ``speaker`` / ``content`` encoder accepts: every reflect-padded conv input must be
+        longer than its padding (models.py:23-28; the same rule avc_* enforces)."""
+        d = self.desc.speaker if which == "speaker" else self.desc.content
+        T = 1
+        while True:
+            Tl, ok = T, T > d.bank_size // 2
+            for l in range(d.n_conv_blocks):
+                ok = ok and Tl > d.kernel_size // 2
+                Tl = -(-Tl // int(d.subsample[l]))
+            if ok:
+                return T
+            T += 1
+
     # ------------------------------------------------------------------------------------------
     def _attack_args(self, kind, vc_tgt, adv_tgt, eps, n_iters, vc_src, w0, inv_norm, want_loss, want_grad, use_graph):
         if kind not in ("emb", "e2e", "fb"):

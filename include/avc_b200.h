@@ -309,6 +309,16 @@ int avc_audio_mel2wav(avc_audio_handle* h, const float* mel, int32_t n_frames, i
  * the rows of one GEMM per transform */
 int avc_audio_wav2mel_batch(avc_audio_handle* h, const float* wav, int32_t B, int64_t n, float* mel, void* stream);
 int avc_audio_mel2wav_batch(avc_audio_handle* h, const float* mel, int32_t B, int32_t n_frames, int32_t n_iter, float* wav, void* stream);
+/* the same for B utterances of ANY lengths laid end to end, in one call: utterance u is samples [s_off[u], s_off[u] + n[u]) of
+ * wav and frames [f_off[u], f_off[u] + F[u]) of mel, F[u] = avc_audio_frames(n[u]) (wav2mel) / n_samples = avc_audio_samples(F[u])
+ * (mel2wav), the offsets being the prefix sums of the host lengths.  All frames are the rows of one GEMM per transform.
+ * mean / std ([n_mels] device fp32, both or neither): wav2mel then writes the speaker-normalised mel (mel - mean) / std, mel2wav
+ * reads x * std + mean (data_utils.py:35-47), both correctly rounded and unfused; NULL keeps the plain mel.  Every length is
+ * validated as by the equal-length calls.  Synchronises the stream. */
+int avc_audio_wav2mel_varlen(avc_audio_handle* h, const float* wav, const int64_t* n_host, int32_t B, const float* mean, const float* std,
+                             float* mel, void* stream);
+int avc_audio_mel2wav_varlen(avc_audio_handle* h, const float* mel, const int32_t* frames_host, int32_t B, int32_t n_iter, const float* mean,
+                             const float* std, float* wav, void* stream);
 int64_t avc_audio_kernel_launches(const avc_audio_handle* h);
 
 /* ---- introspection ----------------------------------------------------------------------- */
