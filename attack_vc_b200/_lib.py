@@ -85,9 +85,19 @@ class AttackArgs(C.Structure):
     ]
 
 
+class AttackVarlenArgs(C.Structure):
+    _fields_ = [
+        ("vc_tgt", C.c_void_p), ("w0", C.c_void_p), ("adv_out", C.c_void_p), ("grad_out", C.c_void_p),
+        ("frames_host", C.POINTER(C.c_int32)), ("B", C.c_int32),
+        ("adv_tgt", C.c_void_p), ("adv_stride", C.c_int64 * 3), ("T_adv", C.c_int32),
+        ("vc_src", C.c_void_p), ("src_stride", C.c_int64 * 3), ("T_src", C.c_int32),
+        ("loss_out", C.c_void_p), ("eps", C.c_float), ("n_iters", C.c_int32), ("inv_norm", C.c_double), ("use_graph", C.c_int32),
+    ]
+
+
 EXPORTS = [
     "avc_create", "avc_destroy", "avc_last_error", "avc_load_weights", "avc_emb_attack", "avc_e2e_attack",
-    "avc_fb_attack", "avc_speaker_encoder", "avc_inference", "avc_decoder_frames", "avc_conv1d_fwd",
+    "avc_fb_attack", "avc_attack_varlen", "avc_speaker_encoder", "avc_inference", "avc_decoder_frames", "avc_conv1d_fwd",
     "avc_conv1d_dgrad", "avc_conv1d_wgrad", "avc_conv1d_wgrad_ex", "avc_instnorm_adain_act_fwd", "avc_instnorm_adain_act_bwd", "avc_adam_tanh_step",
     "avc_unit_timing", "avc_unit_last_ms",
     "avc_kernel_launches", "avc_launches_per_iter", "avc_version",
@@ -134,6 +144,7 @@ def load() -> C.CDLL:
     lib.avc_load_weights.argtypes = [vp, P(WeightView), i32]
     for nm in ("avc_emb_attack", "avc_e2e_attack", "avc_fb_attack"):
         getattr(lib, nm).argtypes = [vp, P(AttackArgs), vp]
+    lib.avc_attack_varlen.argtypes = [vp, i32, P(AttackVarlenArgs), vp]
     lib.avc_attack_begin.argtypes = [vp, i32, P(AttackArgs), vp, P(vp)]
     lib.avc_attack_step.argtypes = [vp, i32, vp]
     lib.avc_attack_end.argtypes = [vp, vp]

@@ -112,6 +112,10 @@ struct TcArgs {
   TcPass pass[kTcMaxPass];
   TcGroup g[kTcMaxPass];
   TcStage st[kTcMaxStages];
+  // Ragged batches (kernels instantiated with VL = true): per-utterance valid rows of the input (T_a), the output (T_y) and
+  // the skip tensor (res.T_r), device int32 [B].  The scalar fields then hold the padded maxima.  Appended last so that the
+  // equal-length kernels keep their parameter offsets.
+  const int* lens_a; const int* lens_y; const int* lens_r;
 };
 
 // ---- host: weight packing ----------------------------------------------------------------------
@@ -231,6 +235,54 @@ __device__ __forceinline__ TcRow tc_row_info(const TcArgs& p, const TcPass& ps, 
     }
   }
   return r;
+}
+
+// Ragged batches: the same with every length read from the utterance's entry of the tables (b is checked against B first:
+// the last tile runs past the batch).  A separate function rather than a branch inside tc_row_info so that the
+// equal-length kernels keep their instruction streams.
+__device__ __forceinline__ TcRow tc_row_info_vl(const TcArgs& p, const TcPass& ps, long long u) {
+  TcRow r;
+  r.b = (int)(u / p.Pv);
+  r.o = ps.so * (int)(u - (long long)r.b * p.Pv) + ps.oo;
+  r.kind = 0; r.t0 = 0; r.t1 = -1; r.rs = 1.f;
+  int T_y = 0;
+  if (r.b < p.B && !(p.dbg & 8)) {
+    T_y = p.lens_y[r.b];
+    if (r.o >= 0 && r.o < T_y) r.kind = 1;
+    else if (p.side && ((r.o < 0 && r.o >= -p.halo_l) || (r.o >= T_y && r.o < T_y + p.halo_r))) {
+      r.kind = 2;
+      r.o = r.o < 0 ? r.o + p.halo_l : p.halo_l + (r.o - T_y);
+    }
+  }
+  if (r.kind == 1) {
+    const int rf = p.res.rf, t = r.o;
+    switch (p.res.mode) {   // the speaker encoder's skip modes
+      case RES_SAME: r.t0 = t; break;
+      case RES_POOL: { const int lo = t * rf, n = min(rf, p.lens_r[r.b] - lo); r.t0 = lo; r.t1 = n > 1 ? lo + 1 : -1; r.rs = 1.f / (float)n; break; }
+      case RES_POOL_BWD: { const int q = rf > 1 ? t >> 1 : t; r.t0 = q; r.rs = 1.f / (float)min(rf, T_y - q * rf); break; }
+      default: break;
+    }
+  }
+  return r;
+}
+
+template <bool VL>
+__device__ __forceinline__ TcRow tc_row(const TcArgs& p, const TcPass& ps, long long u) {
+  if constexpr (VL) return tc_row_info_vl(p, ps, u);
+  else return tc_row_info(p, ps, u);
+}
+
+// Ragged batches: the row of utterance b's input that window position pos reads (reflect padding around the utterance's
+// own length in the forward, zeros outside it in the dgrad), -1 for zeros
+__device__ __forceinline__ int tc_src_row_vl(const TcArgs& p, int b, int pos) {
+  if (b >= p.B) return -1;
+  const int T_a = p.lens_a[b];
+  int rr = pos;
+  if (!p.bwd) {
+    rr = rr < 0 ? -rr : rr;
+    if (rr >= T_a) rr = 2 * (T_a - 1) - rr;
+  }
+  return rr >= 0 && rr < T_a ? rr : -1;
 }
 
 #ifndef AVC_TC_EPI_BATCH
@@ -367,6 +419,7 @@ struct TcDrainProf { long long wait, ld, epi; };
 #else
 #define TCD(x)
 #endif
+template <bool VL>
 __device__ __forceinline__ void tc_drain_and_store(const TcArgs& p, const TcPass& ps, uint32_t tmem_base, uint32_t acc_full0,
                                                    uint32_t acc_empty0, long long v0, int warp, int lane, int& chunk, float* scratch,
                                                    TcDrainProf& dp, int leader_rank = -1) {   // >= 0: acc_empty lives in that CTA of the pair
@@ -378,7 +431,7 @@ __device__ __forceinline__ void tc_drain_and_store(const TcArgs& p, const TcPass
   float acc[NH];
 #pragma unroll
   for (int i = 0; i < NH; ++i) acc[i] = 0.f;
-  const TcRow own = tc_row_info(p, ps, v0 + quad * 32 + lane);   // worked out while the first chunk's MMAs run
+  const TcRow own = tc_row<VL>(p, ps, v0 + quad * 32 + lane);   // worked out while the first chunk's MMAs run
   if (own.kind == 1 && kTcPfDist > 0) {   // the epilogue's operands for this lane's row: into L2 now, read ~20k clk later
     const int c0 = ps.ch_off + half * NH;
     if (p.Om) {
@@ -450,7 +503,9 @@ __device__ __forceinline__ void tc_drain_and_store(const TcArgs& p, const TcPass
 // is what bounds the single-CTA kernel (DESIGN.md).  Cross-CTA protocol: the peer's loader and drain warps arrive on
 // the LEADER's a_full / acc_empty barriers; the peer's warp 1 forwards "my weight half has landed" to the leader's
 // b_fwd barrier; the leader's commits are multicast to the same barrier in both CTAs.
-template <bool PAIR>
+//
+// VL = true: ragged batch, lengths from p.lens_* (see TcArgs).
+template <bool PAIR, bool VL = false>
 __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel_t(const TcArgs p) {
   extern __shared__ __align__(128) unsigned char tc_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -672,13 +727,21 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel_t(const TcArgs p
             const int b = (int)(u / p.Pv);
             const int pos = G.sg * (int)(u - (long long)b * p.Pv) + G.off0;
             int rr = pos;
-            if (!p.bwd) {
-              rr = rr < 0 ? -rr : rr;
-              if (rr >= p.T_a) rr = 2 * (p.T_a - 1) - rr;
-            }
-            if (b < p.B && rr >= 0 && rr < p.T_a && !skip) {
-              src[j] = p.A + (long long)b * p.a_bs + (long long)rr * p.a_rs + G.a_ch_off;
-              if (p.Mk) msk[j] = p.Mk + (long long)b * p.m_bs + (long long)rr * p.m_rs + G.a_ch_off;
+            if constexpr (VL) {
+              rr = tc_src_row_vl(p, b, pos);
+              if (rr >= 0 && !skip) {
+                src[j] = p.A + (long long)b * p.a_bs + (long long)rr * p.a_rs + G.a_ch_off;
+                if (p.Mk) msk[j] = p.Mk + (long long)b * p.m_bs + (long long)rr * p.m_rs + G.a_ch_off;
+              }
+            } else {
+              if (!p.bwd) {
+                rr = rr < 0 ? -rr : rr;
+                if (rr >= p.T_a) rr = 2 * (p.T_a - 1) - rr;
+              }
+              if (b < p.B && rr >= 0 && rr < p.T_a && !skip) {
+                src[j] = p.A + (long long)b * p.a_bs + (long long)rr * p.a_rs + G.a_ch_off;
+                if (p.Mk) msk[j] = p.Mk + (long long)b * p.m_bs + (long long)rr * p.m_rs + G.a_ch_off;
+              }
             }
           }
         }
@@ -770,7 +833,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel_t(const TcArgs p
       const TcPass& ps = p.pass[wk % p.n_pass];
       const long long v0 = tile_row0(wk);
       float* scratch = scr_all + (size_t)(warp - 6) * 32 * kTcScrPitch;
-      tc_drain_and_store(p, ps, tmem_base, acc_full0, acc_empty0, v0, warp, lane, chunk, scratch, dp, PAIR ? 0 : -1);
+      tc_drain_and_store<VL>(p, ps, tmem_base, acc_full0, acc_empty0, v0, warp, lane, chunk, scratch, dp, PAIR ? 0 : -1);
     }
 #ifdef AVC_TC_PROFILE
     if ((p.dbg & 32) && blockIdx.x == 0 && warp == 6 && lane == 0)
@@ -791,9 +854,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel_t(const TcArgs p
 // dgrad: add the extended rows (gradient of the reflect padding) to their mirror rows.
 //   row r' in [1, PL]        += side[PL - r']
 //   row r' in [T-1-PR, T-2]  += side[PL + T - 2 - r']          (both scaled by act'(Om) like the main rows)
+// VL: T is utterance b's own length, lens[b]
+template <bool VL = false>
 __global__ void tc_fold_kernel(float* __restrict__ Y, long long y_bs, int y_rs, const float* __restrict__ side,
                                const float* __restrict__ Om, long long om_bs, int om_rs, float slope,
-                               int B, int T, int N, int PL, int PR) {
+                               int B, int T_max, int N, int PL, int PR, const int* __restrict__ lens) {
   pdl_enter();
   const int n4 = N >> 2, H = PL + PR;
   const long long tot = (long long)B * H * n4;
@@ -801,6 +866,7 @@ __global__ void tc_fold_kernel(float* __restrict__ Y, long long y_bs, int y_rs, 
     const int c = (int)(i % n4) << 2;
     const long long bj = i / n4;
     const int j = (int)(bj % H), b = (int)(bj / H);
+    const int T = VL ? lens[b] : T_max;
     const int r = j < PL ? j + 1 : T - 1 - PR + (j - PL);
     if (r < 0 || r >= T) continue;
     if (j >= PL && r >= 1 && r <= PL) continue;                 // the left-edge thread of this row adds both parts

@@ -51,8 +51,9 @@ inline size_t tc2_smem_bytes() {
 constexpr int kT2DescWords = 5;     // yoff | y2off | g0 | g1 | rs
 // yoff: -1 dead row, <= -2: dgrad halo row at side-buffer offset -2 - yoff; g0 / g1: -1 = none
 
+template <bool VL>
 __device__ __forceinline__ void t2_make_desc(const TcArgs& p, const TcPass& ps, long long u, int* __restrict__ tab, int row) {
-  const TcRow r = tc_row_info(p, ps, u);
+  const TcRow r = tc_row<VL>(p, ps, u);
   int yoff = -1, y2off = 0, g0 = -1, g1 = -1;
   if (r.kind == 2) yoff = -2 - (int)(((long long)r.b * (p.halo_l + p.halo_r) + r.o) * p.side_n);
   if (r.kind == 1) {
@@ -146,6 +147,8 @@ __device__ __forceinline__ void t2_epilogue(const TcArgs& p, uint32_t t_sum, uin
   }
 }
 
+// VL = true: ragged batch, lengths from p.lens_* (see TcArgs).
+template <bool VL = false>
 __global__ void __launch_bounds__(kT2Threads, 1) conv_tc2_kernel(const TcArgs p) {
   extern __shared__ __align__(128) unsigned char t2_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -322,11 +325,17 @@ __global__ void __launch_bounds__(kT2Threads, 1) conv_tc2_kernel(const TcArgs p)
             const int b = (int)(u / p.Pv);
             const int pos = G.sg * (int)(u - (long long)b * p.Pv) + G.off0;
             int rr = pos;
-            if (!p.bwd) {
-              rr = rr < 0 ? -rr : rr;
-              if (rr >= p.T_a) rr = 2 * (p.T_a - 1) - rr;
+            bool ok;
+            if constexpr (VL) {
+              rr = tc_src_row_vl(p, b, pos);
+              ok = rr >= 0;
+            } else {
+              if (!p.bwd) {
+                rr = rr < 0 ? -rr : rr;
+                if (rr >= p.T_a) rr = 2 * (p.T_a - 1) - rr;
+              }
+              ok = b < p.B && rr >= 0 && rr < p.T_a;
             }
-            const bool ok = b < p.B && rr >= 0 && rr < p.T_a;
             rowtab[i] = ok ? (long long)b * p.a_bs + (long long)rr * p.a_rs + G.a_ch_off : -1;
             rowtab[kT2Rows + i] = (ok && p.Mk) ? (long long)b * p.m_bs + (long long)rr * p.m_rs + G.a_ch_off : -1;
           }
@@ -437,7 +446,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) conv_tc2_kernel(const TcArgs p)
       T2P(dq = clock64();)
       asm volatile("bar.sync 2, 256;" ::: "memory");    // the previous tile's epilogue has read its descriptors
       {
-        t2_make_desc(p, ps, v0 + dt, desc, dt);
+        t2_make_desc<VL>(p, ps, v0 + dt, desc, dt);
         const int g0 = desc[2 * kT2N + dt], g1 = desc[3 * kT2N + dt];
         if (kTcPfDist > 0 && g0 >= 0) {                 // the epilogue's operands for this row: into L2 now, read ~20k clk later
           const float* G = p.Om ? p.Om : p.res.R;

@@ -35,6 +35,30 @@ __global__ void layout_out_kernel(const float* __restrict__ src, long long s_bs,
   dst[b * sb + c * sc + t * st] = src[(long long)b * s_bs + (long long)t * s_rs + c];
 }
 
+// packed time-major [sum_b T_b, C] (utterance b's rows start at row offs[b])  <->  [B, T_max, ld] padded time-major:
+// one CTA row per utterance (blockIdx.y), rows past T_b = offs[b+1] - offs[b] are neither read nor written
+__global__ void layout_in_varlen_kernel(const float* __restrict__ src, const int* __restrict__ offs,
+                                        float* __restrict__ dst, long long d_bs, int d_rs, int C) {
+  pdl_enter();
+  const int b = blockIdx.y;
+  const long long r0 = offs[b], n = (long long)(offs[b + 1] - offs[b]) * C;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)(i % C), t = (int)(i / C);
+    dst[(long long)b * d_bs + (long long)t * d_rs + c] = src[r0 * C + i];
+  }
+}
+
+__global__ void layout_out_varlen_kernel(const float* __restrict__ src, long long s_bs, int s_rs, const int* __restrict__ offs,
+                                         float* __restrict__ dst, int C) {
+  pdl_enter();
+  const int b = blockIdx.y;
+  const long long r0 = offs[b], n = (long long)(offs[b + 1] - offs[b]) * C;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)(i % C), t = (int)(i / C);
+    dst[r0 * C + i] = src[(long long)b * s_bs + (long long)t * s_rs + c];
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // InstanceNorm1d(affine=False) + AdaIN + act (+ skip)            (models.py:66-79, 176, 396, 414-431)
 //   out[b,t,c] = act( ((y - mu_bc) * rstd_bc) * std_bc + mean_bc ) + skip
@@ -501,6 +525,7 @@ struct TailArgs {
   float* loss_parts; const int* step; int parts_per_step;
   const float* gemb; int gemb_parts;    // TAIL_BWD without TAIL_LOSS: d emb = sum_p gemb[b][p][128]
   float* gpool;           // [B,128]: d h[b,t,:] for every t (already divided by T_h)
+  const int* lens_h;      // ragged batches (kernels with VL = true): valid rows of h per utterance, device int32 [B]; T_h is their maximum
 };
 
 __device__ __forceinline__ float part_sum(float (*part)[128], int n) {
@@ -510,12 +535,20 @@ __device__ __forceinline__ float part_sum(float (*part)[128], int n) {
   return s;
 }
 
+// rows of h that utterance b pools over
+template <bool VL>
+__device__ __forceinline__ int tail_len(const TailArgs& p, int b) {
+  if constexpr (VL) return p.lens_h[b];
+  else return p.T_h;
+}
+
 constexpr int kTailRing = 3;                       // weight matrices in flight (64 KB each)
 constexpr int kTailSmem = kTailRing * 128 * 128 * 4;
 
 // The chain is 13 dependent 128x128 mat-vecs forward and 13 backward for ONE utterance per CTA: pure
 // latency.  The matrices do not depend on the data, so they stream through a 3-deep ring of bulk copies two
 // layers ahead of the arithmetic (the first two and the biases before the dependency wait).
+template <bool VL = false>
 __global__ void __launch_bounds__(1024) se_tail_kernel(const TailArgs p) {
   extern __shared__ __align__(16) float wring[];    // [kTailRing][128*128]
   __shared__ float part[8][128];
@@ -598,10 +631,10 @@ __global__ void __launch_bounds__(1024) se_tail_kernel(const TailArgs p) {
       const int g = tid >> 7;
       float a = 0.f;
       const float* hb = p.h + (long long)b * p.h_bs + n;
-      for (int t = g; t < p.T_h; t += 8) a += hb[(long long)t * p.h_rs];
+      for (int t = g; t < tail_len<VL>(p, b); t += 8) a += hb[(long long)t * p.h_rs];
       part[g][n] = a;
       __syncthreads();
-      if (tid < 128) { vcur[n] = part_sum(part, n) / (float)p.T_h; va[0][n] = vcur[n]; }
+      if (tid < 128) { vcur[n] = part_sum(part, n) / (float)tail_len<VL>(p, b); va[0][n] = vcur[n]; }
     }
     for (int l = 0; l < p.n_dense; ++l) {
       dense_step(vcur);
@@ -658,7 +691,7 @@ __global__ void __launch_bounds__(1024) se_tail_kernel(const TailArgs p) {
     if (tid < 128) gv[n] = gv[n] + part_sum(part, n);
   }
   __syncthreads();
-  if (tid < 128) p.gpool[(long long)b * 128 + n] = gv[n] / (float)p.T_h;
+  if (tid < 128) p.gpool[(long long)b * 128 + n] = gv[n] / (float)tail_len<VL>(p, b);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -678,6 +711,7 @@ __device__ __forceinline__ void st_cluster_f32(float* local, uint32_t rank, floa
                ::"r"(smem_u32(local)), "r"(rank), "f"(v) : "memory");
 }
 
+template <bool VL = false>
 __global__ void __launch_bounds__(128) se_tail_cluster_kernel(const TailArgs p) {
   extern __shared__ __align__(16) float wsl[];          // [n_all][16][128] this CTA's matrix slices
   __shared__ float recv[2][kTclN][kTclS];
@@ -749,14 +783,14 @@ __global__ void __launch_bounds__(128) se_tail_cluster_kernel(const TailArgs p) 
       const int g = tid >> 4;
       float a = 0.f;
       const float* hb = p.h + (long long)b * p.h_bs + c0 + j;
-      for (int t = g; t < p.T_h; t += 8) a += hb[(long long)t * p.h_rs];
+      for (int t = g; t < tail_len<VL>(p, b); t += 8) a += hb[(long long)t * p.h_rs];
       red[g][j] = a;
       __syncthreads();
       if (tid < kTclS) {
         float s2 = 0.f;
 #pragma unroll
         for (int g2 = 0; g2 < 8; ++g2) s2 += red[g2][j];
-        vcur[j] = s2 / (float)p.T_h; va[0][j] = vcur[j];
+        vcur[j] = s2 / (float)tail_len<VL>(p, b); va[0][j] = vcur[j];
       }
       __syncthreads();
     }
@@ -820,7 +854,7 @@ __global__ void __launch_bounds__(128) se_tail_cluster_kernel(const TailArgs p) 
       if (tid < kTclS) gv[j] = gv[j] + y;
     }
     __syncthreads();
-    if (tid < kTclS) p.gpool[(long long)b * 128 + c0 + j] = gv[j] / (float)p.T_h;
+    if (tid < kTclS) p.gpool[(long long)b * 128 + c0 + j] = gv[j] / (float)tail_len<VL>(p, b);
   }
   cluster_sync_all();      // nobody leaves while a peer may still store into its shared memory
 }

@@ -176,9 +176,11 @@ struct PlanKey {
   long long tc_min_rows = 0;
   float eps = 0.f;
   double inv_norm = 0.0;
+  std::vector<int> frames;   // ragged plans: every utterance's length (empty: equal lengths)
   bool operator==(const PlanKey& o) const {
     return kind == o.kind && B == o.B && T_tgt == o.T_tgt && T_adv == o.T_adv && T_src == o.T_src && use_graph == o.use_graph &&
-           has_grad == o.has_grad && conv_impl == o.conv_impl && tc_min_rows == o.tc_min_rows && eps == o.eps && inv_norm == o.inv_norm;
+           has_grad == o.has_grad && conv_impl == o.conv_impl && tc_min_rows == o.tc_min_rows && eps == o.eps && inv_norm == o.inv_norm &&
+           frames == o.frames;
   }
 };
 
@@ -268,8 +270,11 @@ void init_kernel_attributes() {
   CK(cudaFuncSetAttribute(conv_simt_kernel<1, 8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   CK(cudaFuncSetAttribute(conv_small_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   CK(cudaFuncSetAttribute(conv_small_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CK(cudaFuncSetAttribute(se_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailSmem));
-  CK(cudaFuncSetAttribute(se_tail_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * (2 * kTailMaxDense + 1) * kTclMatBytes > (int)kSmemMax - 4096 ? (int)kSmemMax - 4096 : 2 * (2 * kTailMaxDense + 1) * kTclMatBytes));
+  constexpr int tcl_smem = 2 * (2 * kTailMaxDense + 1) * kTclMatBytes > (int)kSmemMax - 4096 ? (int)kSmemMax - 4096 : 2 * (2 * kTailMaxDense + 1) * kTclMatBytes;
+  CK(cudaFuncSetAttribute(se_tail_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailSmem));
+  CK(cudaFuncSetAttribute(se_tail_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailSmem));
+  CK(cudaFuncSetAttribute(se_tail_cluster_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tcl_smem));
+  CK(cudaFuncSetAttribute(se_tail_cluster_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tcl_smem));
   CK(cudaFuncSetAttribute(norm_act_fwd_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kNormSmemMax));
   CK(cudaFuncSetAttribute(norm_act_fwd_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kNormSmemMax));
   CK(cudaFuncSetAttribute(norm_act_fwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kNormSmemMax));
@@ -278,7 +283,9 @@ void init_kernel_attributes() {
   CK(cudaFuncSetAttribute(norm_act_bwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kNormSmemMax));
   CK(cudaFuncSetAttribute(conv_tc_kernel_t<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   CK(cudaFuncSetAttribute(conv_tc_kernel_t<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CK(cudaFuncSetAttribute(conv_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CK(cudaFuncSetAttribute(conv_tc_kernel_t<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CK(cudaFuncSetAttribute(conv_tc2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CK(cudaFuncSetAttribute(conv_tc2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
 }
 
 // small-M path: every window resident, deep weight ring (conv_simt.cuh: conv_small_kernel)
@@ -433,17 +440,19 @@ bool use_tc2(const TcArgs& t, int sm_count, int tc2) {
   return true;
 }
 
+// t.lens_y set: a ragged batch, run by the VL = true instantiations (never the CTA-pair kernel)
 void launch_conv_tc(const TcArgs& t, int sm_count, cudaStream_t st, int tc2 = 0) {
+  const bool vl = t.lens_y != nullptr;
   if (use_tc2(t, sm_count, tc2)) {
     const long long work = ((t.Mv + kT2N - 1) / kT2N) * t.n_pass;
     dim3 grid((unsigned)std::min<long long>(work, sm_count), 1, 1);   // persistent: one CTA per SM
-    launch_k(conv_tc2_kernel, grid, kT2Threads, tc2_smem_bytes(), st, t);
+    launch_k(vl ? conv_tc2_kernel<true> : conv_tc2_kernel<false>, grid, kT2Threads, tc2_smem_bytes(), st, t);
     return;
   }
   const size_t smem = tc_smem_bytes();
   const long long n_mt = (t.Mv + kTcM - 1) / kTcM;
   static const int pair_env = getenv("AVC_TC_PAIR") ? atoi(getenv("AVC_TC_PAIR")) : 0;
-  if (pair_env && n_mt >= 2) {   // CTA pairs: two M tiles of one pass per cluster, persistent over (tile pair, pass) items
+  if (pair_env && n_mt >= 2 && !vl) {   // CTA pairs: two M tiles of one pass per cluster, persistent over (tile pair, pass) items
     const long long work = ((n_mt + 1) / 2) * t.n_pass;
     dim3 grid(2u * (unsigned)std::min<long long>(work, sm_count / 2), 1, 1);
     launch_k_cluster(2, conv_tc_kernel_t<true>, grid, kTcThreads, smem, st, t);
@@ -451,13 +460,14 @@ void launch_conv_tc(const TcArgs& t, int sm_count, cudaStream_t st, int tc2 = 0)
   }
   const long long work = n_mt * t.n_pass;
   dim3 grid((unsigned)std::min<long long>(work, sm_count), 1, 1);   // persistent: one CTA per SM
-  launch_k(conv_tc_kernel_t<false>, grid, kTcThreads, smem, st, t);
+  launch_k(vl ? conv_tc_kernel_t<false, true> : conv_tc_kernel_t<false>, grid, kTcThreads, smem, st, t);
 }
 
 void launch_tc_fold(const TcArgs& t, int sm_count, cudaStream_t st) {
   const long long n = (long long)t.B * (t.halo_l + t.halo_r) * (t.side_n / 4);
   const unsigned g = (unsigned)std::max(1LL, std::min((n + 255) / 256, (long long)sm_count * 4));
-  launch_k(tc_fold_kernel, g, 256, 0, st, t.Y, t.y_bs, t.y_rs, (const float*)t.side, t.Om, t.om_bs, t.om_rs, t.slope, t.B, t.T_y, t.side_n, t.halo_l, t.halo_r);
+  launch_k(t.lens_y ? tc_fold_kernel<true> : tc_fold_kernel<false>, g, 256, 0, st, t.Y, t.y_bs, t.y_rs, (const float*)t.side, t.Om, t.om_bs,
+           t.om_rs, t.slope, t.B, t.T_y, t.side_n, t.halo_l, t.halo_r, t.lens_y);
 }
 
 // fill the channel groups of a plain Conv1d (forward) -- K split into <=128-channel groups
@@ -508,11 +518,15 @@ int cdiv(int a, int b) { return (a + b - 1) / b; }
 // =================================================================================================
 // emitters: append launches to a vector
 // =================================================================================================
+// per-utterance lengths of a conv in a ragged batch (device int32 [B]): its input, its output and its skip tensor
+struct TcLens { const int* a = nullptr; const int* y = nullptr; const int* r = nullptr; };
+
 struct Emitter {
   avc_handle* h;
   std::vector<Launch>* out;
   Arena* mem;   // scratch that must outlive the launches (dgrad side buffers of the tensor-core path)
-  void conv(const ConvArgs& a, const ConvW* cw = nullptr, const TcOp* multi = nullptr) {
+  // vl.y set: a conv of a ragged batch, which only the tensor-core kernels run
+  void conv(const ConvArgs& a, const ConvW* cw = nullptr, const TcOp* multi = nullptr, TcLens vl = {}) {
     avc_handle* hh = h;
     ConvArgs ac = a;
     double macs = 0;
@@ -523,10 +537,12 @@ struct Emitter {
     Launch l;
     l.kind = LK_CONV; l.flops = 2.0 * macs; l.bytes = bytes;
     TcOp op = multi ? *multi : (cw ? tc_op_conv(*cw, ac.bwd != 0) : TcOp{});
-    if (want_tc(hh, ac, op)) {
+    if (vl.y && !tc_supported(ac, op)) fail(AVC_ERR_INVALID, "ragged attacks run on the tensor-core kernels, which do not support this speaker-encoder conv");
+    if (vl.y || want_tc(hh, ac, op)) {
       const size_t side_n = tc_side_floats(ac);
       float* side = side_n ? mem->f(side_n) : nullptr;
-      const TcArgs t = tc_make_args(ac, op, side, hh->conv_impl == 4 ? 1 : hh->conv_impl == 5 ? 4 : 3);
+      TcArgs t = tc_make_args(ac, op, side, hh->conv_impl == 4 ? 1 : hh->conv_impl == 5 ? 4 : 3);
+      t.lens_a = vl.a; t.lens_y = vl.y; t.lens_r = vl.r;
       const int smc0 = hh->sm_count;
       const int tc2 = hh->conv_impl == 6 ? 2 : hh->conv_impl == 7 ? 1 : 0;      // 6: N = 256 kernel everywhere, 7: N = 128 kernel everywhere
       l.fn = [t, smc0, tc2](cudaStream_t st) { launch_conv_tc(t, smc0, st, tc2); };
@@ -642,10 +658,22 @@ struct EncActs {
   float *tail_acts = nullptr, *emb = nullptr, *gpool = nullptr;
   // backward scratch
   float *gA = nullptr, *gB = nullptr, *gH = nullptr, *gcat = nullptr, *gin = nullptr;
+  // ragged batch (speaker encoder only): lens[l][b] = valid rows of utterance b at level l (device), Tl[l] their maximum.
+  // Null for equal lengths.
+  const int* lens[AVC_MAX_BLOCKS + 1]{};
+  TcLens vl(int la, int ly, int lr = -1) const { return lens[0] ? TcLens{lens[la], lens[ly], lr >= 0 ? lens[lr] : nullptr} : TcLens{}; }
   Tens input(const EncoderW& W) const {
     return Tens{cat + W.n_bank * W.d.c_bank, (long long)T * W.c_cat, W.c_cat, T};
   }
 };
+
+// reflect padding needs pad < length for every conv INPUT (PyTorch raises otherwise, models.py:23-28): the bank sees T,
+// both convs of block l see Tl[l]; the length after the last sub-sampling only feeds the pooling
+bool too_short_for_encoder(const EncoderW& W, int T) {
+  bool too_short = T <= W.d.bank_size / 2;
+  for (int l = 0, t = T; l < W.d.n_conv_blocks; t = cdiv(t, W.d.subsample[l]), ++l) too_short = too_short || t <= W.d.kernel_size / 2;
+  return too_short;
+}
 
 EncActs alloc_encoder(Arena& m, const EncoderW& W, int B, int T, bool need_bwd, bool content) {
   EncActs A;
@@ -653,11 +681,7 @@ EncActs alloc_encoder(Arena& m, const EncoderW& W, int B, int T, bool need_bwd, 
   const int ch = W.d.c_h;
   A.Tl[0] = T;
   for (int l = 0; l < W.d.n_conv_blocks; ++l) A.Tl[l + 1] = cdiv(A.Tl[l], W.d.subsample[l]);
-  // reflect padding needs pad < length for every conv INPUT (PyTorch raises otherwise, models.py:23-28): the bank sees T,
-  // both convs of block l see Tl[l]; the length after the last sub-sampling only feeds the pooling
-  bool too_short = T <= W.d.bank_size / 2;
-  for (int l = 0; l < W.d.n_conv_blocks; ++l) too_short = too_short || A.Tl[l] <= W.d.kernel_size / 2;
-  if (too_short) fail(AVC_ERR_INVALID, "utterance of %d frames is too short for reflect padding", T);
+  if (too_short_for_encoder(W, T)) fail(AVC_ERR_INVALID, "utterance of %d frames is too short for reflect padding", T);
   A.cat = m.f((size_t)B * T * W.c_cat);
   A.h0 = m.f((size_t)B * T * ch);
   for (int l = 0; l < W.d.n_conv_blocks; ++l) {
@@ -702,13 +726,13 @@ void emit_bank_and_inconv(Emitter& E, const EncoderW& W, const EncActs& A, bool 
       tc_ok = tc_ok && gi >= 0 && op.add_pass(gi, gi + 1, pk.cn[0], z * W.d.c_bank, 1, 0);   // one pass per bank conv
     }
     if (!tc_ok) op = TcOp{};
-    E.conv(a, nullptr, &op);
+    E.conv(a, nullptr, &op, A.vl(0, 0));
   }
   {   // 1x1 in-conv over the concatenation (models.py:192 / :337)
     Tens cat{A.cat, x.bs, W.c_cat, A.T};
     Tens outT = tens(content ? A.tmp : A.h0, A.T, W.d.c_h);
     ConvArgs a = fwd_conv_args(W.in_conv, cat, outT, A.B, !content, slope);
-    E.conv(a, &W.in_conv);
+    E.conv(a, &W.in_conv, nullptr, A.vl(0, 0));
     if (content) emit_norm_fwd(E, A.tmp, A.B, A.T, W.d.c_h, nullptr, 0, nullptr, nullptr, A.h0, no_res(), slope);
   }
 }
@@ -723,11 +747,11 @@ void emit_encoder_blocks_fwd(Emitter& E, const EncoderW& W, const EncActs& A, bo
     ResArgs res = mk_res(in, sub > 1 ? RES_POOL : RES_SAME, sub);
     if (!content) {
       ConvArgs a1 = fwd_conv_args(W.c1[l], in, tens(A.h1[l], Ti, ch), A.B, true, slope);
-      E.conv(a1, &W.c1[l]);
+      E.conv(a1, &W.c1[l], nullptr, A.vl(l, l));
       ConvArgs a2 = fwd_conv_args(W.c2[l], tens(A.h1[l], Ti, ch), tens(A.hout[l], To, ch), A.B, true, slope);
       a2.Y2 = A.h2[l]; a2.y2_bs = (long long)To * ch; a2.y2_rs = ch;
       a2.res = res;
-      E.conv(a2, &W.c2[l]);
+      E.conv(a2, &W.c2[l], nullptr, A.vl(l, l + 1, l));
     } else {
       ConvArgs a1 = fwd_conv_args(W.c1[l], in, tens(A.tmp, Ti, ch), A.B, false, slope);
       E.conv(a1, &W.c1[l]);
@@ -752,6 +776,7 @@ TailArgs tail_args(const EncoderW& W, const EncActs& A) {
   t.Wto = W.Wto; t.Wo = W.Wo; t.bo = W.bo;
   t.slope = W.d.neg_slope;
   t.acts = A.tail_acts; t.emb = A.emb; t.gpool = A.gpool;
+  t.lens_h = A.lens[nb];
   return t;
 }
 
@@ -761,9 +786,10 @@ void emit_tail(Emitter& E, const TailArgs& t, int B) {
   const size_t csm = (size_t)n_mats * kTclMatBytes;
   static const bool no_cluster = getenv("AVC_NO_TAIL_CLUSTER") != nullptr;
   const bool cluster = !no_cluster && B * kTclN <= E.h->sm_count && csm + 4096 <= kSmemMax;
-  E.push(LK_TAIL, 2.0 * B * 128 * 128 * (2 * t.n_dense + 1) * (((t.mode & TAIL_FWD) ? 1 : 0) + ((t.mode & TAIL_BWD) ? 1 : 0)), 0, [t, B, cluster, csm](cudaStream_t st) {
-    if (cluster) launch_k_cluster(kTclN, se_tail_cluster_kernel, B * kTclN, 128, csm, st, t);
-    else launch_k(se_tail_kernel, B, 1024, kTailSmem, st, t);
+  const bool vl = t.lens_h != nullptr;
+  E.push(LK_TAIL, 2.0 * B * 128 * 128 * (2 * t.n_dense + 1) * (((t.mode & TAIL_FWD) ? 1 : 0) + ((t.mode & TAIL_BWD) ? 1 : 0)), 0, [t, B, cluster, csm, vl](cudaStream_t st) {
+    if (cluster) launch_k_cluster(kTclN, vl ? se_tail_cluster_kernel<true> : se_tail_cluster_kernel<false>, B * kTclN, 128, csm, st, t);
+    else launch_k(vl ? se_tail_kernel<true> : se_tail_kernel<false>, B, 1024, kTailSmem, st, t);
   });
 }
 
@@ -785,12 +811,12 @@ void emit_speaker_bwd(Emitter& E, const EncoderW& W, const EncActs& A, const Ten
     ConvArgs a2 = bwd_conv_args(W.c2[l], gout, gH, A.B, slope);
     a2.Mk = A.h2[l]; a2.m_bs = (long long)To * ch; a2.m_rs = ch;
     a2.Om = A.h1[l]; a2.om_bs = (long long)Ti * ch; a2.om_rs = ch;
-    E.conv(a2, &W.c2[l]);
+    E.conv(a2, &W.c2[l], nullptr, A.vl(l + 1, l));
     // through the first conv, plus the skip path (avg-pool backward when sub-sampled)
     Tens gx = tens(pingpong[l & 1], Ti, ch);
     ConvArgs a1 = bwd_conv_args(W.c1[l], gH, gx, A.B, slope);
     a1.res = mk_res(gout, sub > 1 ? RES_POOL_BWD : RES_SAME, sub);
-    E.conv(a1, &W.c1[l]);
+    E.conv(a1, &W.c1[l], nullptr, A.vl(l, l, l + 1));
     gout = gx;
   }
   if (nb == 0) fail(AVC_ERR_INVALID, "n_conv_blocks must be > 0");
@@ -803,7 +829,8 @@ void emit_speaker_bwd(Emitter& E, const EncoderW& W, const EncActs& A, const Ten
     // planes by one elementwise pass and conv2d_tc_kernel streams both operands with TMA tensor loads (3xTF32).
     static const bool no_tma = getenv("AVC_NO_TMA_INCONV") != nullptr;
     const bool contiguous = gout.rs == ch && gout.bs == (long long)A.T * ch;
-    if (!no_tma && W.in_conv.fwd_h && contiguous && ch % 32 == 0 && want_tc(E.h, a, tc_op_conv(W.in_conv, true))) {
+    // (ragged batches too: a 1x1 GEMM over the padded rows, whose dead rows only reach dead rows of gcat)
+    if (!no_tma && W.in_conv.fwd_h && contiguous && ch % 32 == 0 && (A.lens[0] || want_tc(E.h, a, tc_op_conv(W.in_conv, true)))) {
       const size_t n = (size_t)A.B * A.T * ch;
       float* ph = E.mem->f(n); float* pl = E.mem->f(n);
       const float* g = gout.p; const float* mk = A.h0;
@@ -824,7 +851,7 @@ void emit_speaker_bwd(Emitter& E, const EncoderW& W, const EncActs& A, const Ten
         launch_conv2d_tc(X, wh, wl, ch, rows, c, smc, st, 1);
       });
     } else {
-      E.conv(a, &W.in_conv);
+      E.conv(a, &W.in_conv, nullptr, A.vl(0, 0));
     }
   }
   {   // conv bank: sum of the 8 transposed convs of (gcat_k * act'(cat_k)) + pass-through slice
@@ -850,7 +877,7 @@ void emit_speaker_bwd(Emitter& E, const EncoderW& W, const EncActs& A, const Ten
     tc_ok = tc_ok && op.add_pass(0, op.n_groups, W.bank[0].tc_bwd[0].cn[0], 0, 1, -PL);   // one pass sums the 8 transposed convs
     if (!tc_ok) op = TcOp{};
     static const bool no_zk = getenv("AVC_NO_KSPLIT") != nullptr;
-    if (parts && !no_zk && W.n_bank >= kMaxZk && !want_tc(E.h, a, op) && E.small_tm_of(a, nullptr)) {
+    if (parts && !no_zk && !A.lens[0] && W.n_bank >= kMaxZk && !want_tc(E.h, a, op) && E.small_tm_of(a, nullptr)) {
       // batch-1 plans: this conv contracts K = sum_k k*c_bank (36 weight slabs for the 8-kernel bank), four times the longest
       // other layer, on too few CTAs.  Split K into kMaxZk balanced ranges of whole groups (longest-processing-time first).
       ConvArgs sp = a;
@@ -879,7 +906,7 @@ void emit_speaker_bwd(Emitter& E, const EncoderW& W, const EncActs& A, const Ten
         return;
       }
     }
-    E.conv(a, nullptr, &op);
+    E.conv(a, nullptr, &op, A.vl(0, 0, 0));
   }
 }
 
@@ -1190,6 +1217,22 @@ void emit_layout_out_io(Emitter& E, const Tens& src, float* const* dst, const in
     launch_k(layout_out_kernel, (unsigned)((n + 255) / 256), 256, 0, st, d.p, d.bs, d.rs, *dst, (long long)s[0], (long long)s[1], (long long)s[2], B, C, d.T);
   });
 }
+// ragged batches: the caller's packed [sum_b T_b, C] (row offsets `offs`, device [B+1]) <-> the padded slots of dst / src
+void emit_layout_in_varlen_io(Emitter& E, const float* const* src, const int* offs, const Tens& dst, int B, int C, long long rows) {
+  const Tens d = dst;
+  const unsigned gx = (unsigned)cdiv(d.T * C, 256);
+  E.push(LK_LAYOUT, 0, 8.0 * rows * C, [=](cudaStream_t st) {
+    launch_k(layout_in_varlen_kernel, dim3(gx, B), 256, 0, st, *src, offs, d.p, d.bs, d.rs, C);
+  });
+}
+void emit_layout_out_varlen_io(Emitter& E, const Tens& src, const int* offs, float* const* dst, int B, int C, long long rows) {
+  const Tens d = src;
+  const unsigned gx = (unsigned)cdiv(d.T * C, 256);
+  E.push(LK_LAYOUT, 0, 8.0 * rows * C, [=](cudaStream_t st) {
+    if (!*dst) return;
+    launch_k(layout_out_varlen_kernel, dim3(gx, B), 256, 0, st, (const float*)d.p, d.bs, d.rs, offs, *dst, C);
+  });
+}
 void emit_copy(Emitter& E, float* dst, const float* src, size_t n) {
   E.push(LK_COPY, 0, 8.0 * n, [=](cudaStream_t st) { CK(cudaMemcpyAsync(dst, src, n * sizeof(float), cudaMemcpyDeviceToDevice, st)); });
 }
@@ -1384,7 +1427,21 @@ void capture_iters(Plan& plan, int reps, cudaGraph_t* g, cudaGraphExec_t* x) {
   CK(cudaGraphInstantiate(x, *g, 0));
 }
 
-std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st) {
+// Ragged batches (avc_attack_varlen): the perturbed utterances differ in length.  Only the speaker encoder on the perturbed
+// batch (se1) sees them: its activations keep the padded layout [B, Tl[l], C] with Tl[l] the longest utterance's rows and
+// a device table of every utterance's rows per level; rows past an utterance's length are dead -- no conv reads them for a
+// live row or stores them, and the arena's zero-initialised slabs keep them 0 in the optimiser state and the perturbed
+// input.  Every speaker-encoder conv of se1 runs on the tensor-core kernels, whatever its row count.
+void check_ragged_lengths(const avc_handle* h, const std::vector<int>& frames) {
+  for (size_t b = 0; b < frames.size(); ++b)
+    if (frames[b] <= 0 || too_short_for_encoder(h->se, frames[b]))
+      fail(AVC_ERR_INVALID, "utterance %zu of %d frames is too short for the speaker encoder's reflect padding", b, frames[b]);
+}
+
+// frames: per-utterance lengths of a ragged batch (a->vc_tgt, w0, adv_out, grad_out are then packed [sum T_b, C] and
+// a->T_tgt is the longest), nullptr for equal lengths
+std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st,
+                                   const std::vector<int>* frames = nullptr) {
   if (!h->have_weights) fail(AVC_ERR_STATE, "avc_load_weights must be called before an attack");
   if (!a || !a->vc_tgt || !a->adv_tgt || !a->w0 || !a->adv_out) fail(AVC_ERR_INVALID, "null tensor argument");
   if (kind != K_EMB && !a->vc_src) fail(AVC_ERR_INVALID, "vc_src is required for e2e and fb attacks");
@@ -1425,6 +1482,26 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
   EncActs se1 = alloc_encoder(m, SE, B, T, true, false);
   const Tens adv = se1.input(SE);   // the perturbed utterance lives in the bank concat buffer
   Tens xT = tens(x, T, C), wT = tens(w, T, C);
+  const bool ragged = frames != nullptr;
+  const int* offs = nullptr;        // ragged: row offsets of the packed caller tensors, device [B+1]
+  long long rows = (long long)B * T;
+  if (ragged) {
+    std::vector<int> o(B + 1, 0), len(frames->begin(), frames->end());
+    for (int b = 0; b < B; ++b) o[b + 1] = o[b] + len[b];
+    rows = o[B];
+    offs = m.upload(o);
+    for (int l = 0; l <= SE.d.n_conv_blocks; ++l) {
+      se1.lens[l] = m.upload(len);
+      if (l < SE.d.n_conv_blocks) for (int& t : len) t = cdiv(t, SE.d.subsample[l]);
+    }
+  }
+  // the caller's utterance-shaped tensors: [B, C, T] strided, or packed [sum T_b, C] in a ragged batch
+  auto utt_in = [&](Emitter& E, const float* const* src, const int64_t* s, const Tens& dst) {
+    if (ragged) emit_layout_in_varlen_io(E, src, offs, dst, B, C, rows);
+    else emit_layout_in_io(E, src, s, dst, B, C);
+  };
+  // a ragged batch takes the adversarial target through its own (equal-length) encoder pass even when T_adv == T_tgt
+  const bool adv_in_se1 = !ragged && a->T_adv == T;
   {   // a (possibly reused) plan starts from a fresh optimiser: m = v = 0, step 0
     float* mz = mm; float* vz = vv; int* sz = step; unsigned int* dz = done;
     S.push(LK_COPY, 0, 8.0 * nel, [=](cudaStream_t s_) {
@@ -1432,8 +1509,8 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
       CK(cudaMemsetAsync(sz, 0, sizeof(int), s_)); CK(cudaMemsetAsync(dz, 0, sizeof(unsigned int), s_));
     });
   }
-  emit_layout_in_io(S, &io->vc_tgt, io->tgt_stride, xT, B, C);
-  emit_layout_in_io(S, &io->w0, io->w0_stride, wT, B, C);
+  utt_in(S, &io->vc_tgt, io->tgt_stride, xT);
+  utt_in(S, &io->w0, io->w0_stride, wT);
 
   float* org = nullptr;   // targets
   float* tgt = nullptr;
@@ -1472,9 +1549,9 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
     org = m.f((size_t)B * 128);
     tgt = m.f((size_t)B * 128);
     // targets (attack_utils.py:73-75)
-    emit_layout_in_io(S, &io->vc_tgt, io->tgt_stride, adv, B, C);
+    utt_in(S, &io->vc_tgt, io->tgt_stride, adv);
     se_forward(S, se1, TAIL_FWD, nullptr, nullptr, org);
-    if (a->T_adv == T) {
+    if (adv_in_se1) {
       emit_layout_in_io(S, &io->adv_tgt, io->adv_stride, adv, B, C);
       se_forward(S, se1, TAIL_FWD, nullptr, nullptr, tgt);
     } else {
@@ -1519,11 +1596,11 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
       parts = (int)mg;
       loss_parts = m.f((size_t)std::max(n_iters, 1) * parts);
       // targets (attack_utils.py:35-37)
-      emit_layout_in_io(S, &io->vc_tgt, io->tgt_stride, adv, B, C);
+      utt_in(S, &io->vc_tgt, io->tgt_stride, adv);
       se_forward(S, se1, TAIL_FWD, nullptr, nullptr, nullptr);
       emit_decoder_fwd(S, h->dec, dec, se1.emb, doutT);
       emit_copy(S, org, dout, nout);
-      if (a->T_adv == T) {
+      if (adv_in_se1) {
         emit_layout_in_io(S, &io->adv_tgt, io->adv_stride, adv, B, C);
         se_forward(S, se1, TAIL_FWD, nullptr, nullptr, nullptr);
         emit_decoder_fwd(S, h->dec, dec, se1.emb, doutT);
@@ -1552,11 +1629,11 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
       EncActs se2 = alloc_encoder(m, SE, B, T_dec, true, false);   // speaker encoder on the converted utterance
       const Tens conv_out = se2.input(SE);
       // targets (attack_utils.py:117-119)
-      emit_layout_in_io(S, &io->vc_tgt, io->tgt_stride, adv, B, C);
+      utt_in(S, &io->vc_tgt, io->tgt_stride, adv);
       se_forward(S, se1, TAIL_FWD, nullptr, nullptr, nullptr);
       emit_decoder_fwd(S, h->dec, dec, se1.emb, conv_out);
       se_forward(S, se2, TAIL_FWD, nullptr, nullptr, org);
-      if (a->T_adv == T) {
+      if (adv_in_se1) {
         emit_layout_in_io(S, &io->adv_tgt, io->adv_stride, adv, B, C);
         se_forward(S, se1, TAIL_FWD, nullptr, nullptr, tgt);
       } else {
@@ -1586,7 +1663,8 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
   }
 
   // ---- finish: result, loss curve, last gradient -----------------------------------------------
-  emit_layout_out_io(F, adv, &io->adv_out, io->out_stride, B, C);
+  if (ragged) emit_layout_out_varlen_io(F, adv, offs, &io->adv_out, B, C, rows);
+  else emit_layout_out_io(F, adv, &io->adv_out, io->out_stride, B, C);
   {
     float* lp = loss_parts; const int pp = parts;
     F.push(LK_LOSS, 0, 4.0 * pp * n_iters, [=](cudaStream_t s_) {
@@ -1594,7 +1672,13 @@ std::unique_ptr<Plan> build_attack(avc_handle* h, AttackKind kind, const avc_att
       if (io->loss_out && n > 0) launch_k(loss_sum_kernel, (n + 127) / 128, 128, 0, s_, (const float*)lp, pp, n, io->loss_out);
     });
   }
-  if (gw) {
+  if (gw && ragged) {
+    const Tens g = tens(gw, T, C);
+    F.push(LK_LAYOUT, 0, 8.0 * rows * C, [=](cudaStream_t s_) {
+      if (io->grad_out && io->n_iters > 0)
+        launch_k(layout_out_varlen_kernel, dim3((unsigned)cdiv(T * C, 256), B), 256, 0, s_, (const float*)g.p, g.bs, g.rs, offs, io->grad_out, C);
+    });
+  } else if (gw) {
     const long long cs0 = (long long)C * T, cs1 = T;
     const Tens g = tens(gw, T, C);
     const long long n = (long long)B * T * C;
@@ -1893,9 +1977,10 @@ void finish_attack(avc_handle* h, Plan& plan, cudaStream_t st) {
 }
 
 // ---- plan cache ------------------------------------------------------------------------------------------
-PlanKey make_key(const avc_handle* h, int kind, const avc_attack_args* a) {
+PlanKey make_key(const avc_handle* h, int kind, const avc_attack_args* a, const std::vector<int>* frames) {
   PlanKey k;
   if (!a) return k;
+  if (frames) k.frames = *frames;
   k.kind = kind; k.B = a->B; k.T_tgt = a->T_tgt; k.T_adv = a->T_adv; k.T_src = kind == K_EMB ? 0 : a->T_src;
   k.use_graph = a->use_graph != 0; k.has_grad = a->grad_out != nullptr; k.conv_impl = h->conv_impl; k.tc_min_rows = h->tc_min_rows;
   k.eps = a->eps; k.inv_norm = a->inv_norm > 0 ? a->inv_norm : 0.0;
@@ -1924,8 +2009,9 @@ void put_cached(avc_handle* h, std::unique_ptr<Plan> plan) {
 }
 
 // a plan ready to iterate: a cached one rebound to this call's tensors (its setup re-run), else a new one
-std::unique_ptr<Plan> acquire_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st) {
-  const PlanKey key = make_key(h, (int)kind, a);
+std::unique_ptr<Plan> acquire_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st,
+                                     const std::vector<int>* frames = nullptr) {
+  PlanKey key = make_key(h, (int)kind, a, frames);
   std::unique_ptr<Plan> plan = a ? take_cached(h, key, a->n_iters) : nullptr;
   if (plan) {
     if (!a->vc_tgt || !a->adv_tgt || !a->w0 || !a->adv_out || (kind != K_EMB && !a->vc_src)) fail(AVC_ERR_INVALID, "null tensor argument");
@@ -1942,17 +2028,17 @@ std::unique_ptr<Plan> acquire_attack(avc_handle* h, AttackKind kind, const avc_a
     h->launches_per_iter = (int)plan->iter.size();
     return plan;
   }
-  plan = build_attack(h, kind, a, st);
-  plan->key = key;
+  plan = build_attack(h, kind, a, st, frames);
+  plan->key = std::move(key);
   return plan;
 }
 
-void run_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st) {
+void run_attack(avc_handle* h, AttackKind kind, const avc_attack_args* a, cudaStream_t st, const std::vector<int>* frames = nullptr) {
   static const bool timing = getenv("AVC_TIMING") != nullptr;   // host-side phase times on stderr
   auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t0 = now();
   const long long hits0 = h->plan_cache_hits;
-  std::unique_ptr<Plan> plan = acquire_attack(h, kind, a, st);
+  std::unique_ptr<Plan> plan = acquire_attack(h, kind, a, st, frames);
   const double t1 = now();
   step_attack(h, *plan, a->n_iters, st);
   const double t2 = now();
@@ -2083,6 +2169,26 @@ int avc_e2e_attack(avc_handle* h, const avc_attack_args* a, void* stream) {
 int avc_fb_attack(avc_handle* h, const avc_attack_args* a, void* stream) {
   if (!h) return AVC_ERR_INVALID;
   return guarded(h, [&] { run_attack(h, K_FB, a, (cudaStream_t)stream); });
+}
+
+int avc_attack_varlen(avc_handle* h, int32_t kind, const avc_attack_varlen_args* v, void* stream) {
+  if (!h) return AVC_ERR_INVALID;
+  return guarded(h, [&] {
+    if (kind < 0 || kind > 2) fail(AVC_ERR_INVALID, "kind must be 0 (emb), 1 (e2e) or 2 (fb)");
+    if (!v || !v->frames_host || v->B <= 0) fail(AVC_ERR_INVALID, "null argument or B <= 0");
+    if (h->conv_impl == 1 || h->conv_impl == 3)
+      fail(AVC_ERR_INVALID, "ragged attacks run on the tensor-core kernels (AVC_CONV_IMPL=%d selects the CUDA cores)", h->conv_impl);
+    std::vector<int> frames(v->frames_host, v->frames_host + v->B);
+    check_ragged_lengths(h, frames);
+    avc_attack_args a{};
+    a.vc_tgt = v->vc_tgt; a.B = v->B; a.T_tgt = *std::max_element(frames.begin(), frames.end());
+    a.adv_tgt = v->adv_tgt; a.T_adv = v->T_adv;
+    a.vc_src = v->vc_src; a.T_src = v->T_src;
+    for (int i = 0; i < 3; ++i) { a.adv_stride[i] = v->adv_stride[i]; a.src_stride[i] = v->src_stride[i]; }
+    a.w0 = v->w0; a.adv_out = v->adv_out; a.loss_out = v->loss_out; a.grad_out = v->grad_out;
+    a.eps = v->eps; a.n_iters = v->n_iters; a.inv_norm = v->inv_norm; a.use_graph = v->use_graph;
+    run_attack(h, (AttackKind)kind, &a, (cudaStream_t)stream, &frames);
+  });
 }
 
 int avc_attack_begin(avc_handle* h, int32_t kind, const avc_attack_args* a, void* stream, avc_session** out) {

@@ -136,6 +136,12 @@ struct Arena {
     else CK(cudaMemcpy(p, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice));
     return p;
   }
+  int* upload(const std::vector<int>& v) {
+    int* p = raw<int>(v.size());
+    if (ordered) CK(cudaMemcpyAsync(p, v.data(), v.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
+    else CK(cudaMemcpy(p, v.data(), v.size() * sizeof(int), cudaMemcpyHostToDevice));
+    return p;
+  }
   ~Arena() {
     for (auto& s : slabs) {
       if (pool) pool->give(s.first, s.second); else cudaFree(s.first);

@@ -7,7 +7,8 @@ Per utterance the reference runs ``file2mel`` -> ``normalize`` with the checkpoi
 * ONE ragged front-end call (``avc_audio_wav2mel_varlen``, normalisation fused) over every target utterance plus the
   attack target and the conversion source;
 * one ``Engine.attack`` per chunk of equal-length utterances (``group_by_length``; at most ``max_batch[kind]`` per chunk),
-  each utterance with the normaliser a single ``attack.py`` run gives it, so that batching changes no result;
+  each utterance with the normaliser a single ``attack.py`` run gives it, so that batching changes no result -- or, with
+  ``mixed_lengths=True``, one ``Engine.attack_varlen`` per chunk of the utterances sorted by length (``plan_sorted_chunks``);
 * ONE ragged back-end call (``avc_audio_mel2wav_varlen``, denormalisation fused) over every defended mel.
 
 ``librosa.load``, trimming and ``sf.write`` stay with the caller, as in ``audio.py``.  PyTorch allocates, copies and
@@ -40,6 +41,16 @@ def plan_chunks(frames: Sequence[int], max_batch: int) -> List[Tuple[int, List[i
         for i in range(0, len(idx), max_batch):
             out.append((T, idx[i:i + max_batch]))
     return out
+
+
+def plan_sorted_chunks(frames: Sequence[int], max_batch: int) -> List[List[int]]:
+    """Ragged attack calls for utterances of ``frames[i]`` frames: the input indices sorted by length, longest first (ties
+    in input order), cut into runs of at most ``max_batch`` -> [[input indices], ...].  Neighbours in the sorted order
+    have similar lengths, so a chunk's padded rows stay few."""
+    if max_batch < 1:
+        raise ValueError(f"max_batch must be >= 1 (got {max_batch})")
+    order = sorted(range(len(frames)), key=lambda i: -int(frames[i]))
+    return [order[i:i + max_batch] for i in range(0, len(order), max_batch)]
 
 
 def utterance_inv_norm(kind: str, c_emb: int, c_mel: int, T_out: int) -> float:
@@ -115,14 +126,18 @@ class Defender:
 
     # ---- the defence ---------------------------------------------------------------------------------------------
     def defend(self, vc_tgt: Sequence[Tensor], adv_tgt: Tensor, attack_type: str = "emb", eps: float = 0.1, n_iters: int = 1500,
-               vc_src: Optional[Tensor] = None, griffin_lim_iters: int = 100, return_mels: bool = False):
+               vc_src: Optional[Tensor] = None, griffin_lim_iters: int = 100, return_mels: bool = False, mixed_lengths: bool = False):
         """attack.py on every waveform of ``vc_tgt`` (trimmed, on the device) against the one attack target ``adv_tgt``
         (and conversion source ``vc_src`` for e2e / fb).  Defaults as attack.py:95-113: emb attack, eps 0.1, 1500
         iterations; griffin_lim's 100 iterations (data_utils.py:173).  Returns the defended waveforms in input order, and
         with ``return_mels`` also the defended normalised mels ([n_frames, 80] each): ``(wavs, mels)``.
 
         Seeded like attack.py run on each file in turn: the initial noise of utterance i is drawn, in input order, exactly
-        as attack_utils draws it for that utterance alone."""
+        as attack_utils draws it for that utterance alone.
+
+        ``mixed_lengths``: attack chunks of the utterances sorted by length, each one ragged ``Engine.attack_varlen`` on the
+        tensor-core kernels, instead of one ``Engine.attack`` per chunk of equal-length utterances.  Fewer, larger attack
+        calls when few utterances share a length; same results bit for bit when both run on the same kernels."""
         kind = attack_type
         if kind not in KINDS:
             raise ValueError(f"attack_type must be one of {KINDS} (got {kind!r})")
@@ -144,9 +159,12 @@ class Defender:
         ev = _StageEvents(self.device)
         self._events = ev
         ev.record(0)
-        # 1. front-end: the targets in chunk order, so that every chunk's mels are one contiguous [B_g, T, 80] block
-        chunks = plan_chunks(frames, int(self.max_batch[kind]))
-        order = [i for _, idx in chunks for i in idx]
+        # 1. front-end: the targets in chunk order, so that every chunk's mels are one contiguous block
+        if mixed_lengths:
+            chunks = plan_sorted_chunks(frames, int(self.max_batch[kind]))
+        else:
+            chunks = [idx for _, idx in plan_chunks(frames, int(self.max_batch[kind]))]
+        order = [i for idx in chunks for i in idx]
         extra = [adv] + ([src] if src is not None else [])
         mels = self.wav2mel([tgts[i] for i in order] + extra)
         adv_mel = mels[len(order)]
@@ -158,9 +176,9 @@ class Defender:
         inv = utterance_inv_norm(kind, self.engine.c_emb, self.n_mels, self.engine.decoder_frames(T_src) if kind == "e2e" else 0)
         out: List[Optional[Tensor]] = [None] * len(tgts)
         pos = 0
-        for T, idx in chunks:
-            out_chunk = self._attack_chunk(kind, mels[pos:pos + len(idx)], [w0[i] for i in idx], adv_mel, src_mel, eps,
-                                           int(n_iters), inv)
+        attack_chunk = self._attack_ragged if mixed_lengths else self._attack_chunk
+        for idx in chunks:
+            out_chunk = attack_chunk(kind, mels[pos:pos + len(idx)], [w0[i] for i in idx], adv_mel, src_mel, eps, int(n_iters), inv)
             for k, i in enumerate(idx):
                 out[i] = out_chunk[k]
             pos += len(idx)
@@ -193,6 +211,15 @@ class Defender:
         vs = src_mel.t().unsqueeze(0).expand(B, -1, -1) if src_mel is not None else None
         res = self.engine.attack(kind, blk, at, eps, n_iters, vc_src=vs, w0=w, inv_norm=inv_norm)
         return [res[k].t() for k in range(B)]
+
+    def _attack_ragged(self, kind: str, mels: Sequence[Tensor], w0: Sequence[Tensor], adv_mel: Tensor, src_mel: Optional[Tensor],
+                       eps: float, n_iters: int, inv_norm: float) -> List[Tensor]:
+        """One Engine.attack_varlen over utterances of any lengths whose [T_i, 80] mels lie end to end in one buffer ->
+        the defended [T_i, 80] mels (views of one packed output)."""
+        B = len(mels)
+        at = adv_mel.t().unsqueeze(0).expand(B, -1, -1)            # batch stride 0
+        vs = src_mel.t().unsqueeze(0).expand(B, -1, -1) if src_mel is not None else None
+        return self.engine.attack_varlen(kind, mels, at, eps, n_iters, vc_src=vs, w0=[wk[0].t() for wk in w0], inv_norm=inv_norm)
 
     @property
     def last_stage_ms(self) -> Dict[str, float]:

@@ -10,13 +10,13 @@ the RNG draw of w0 and the CUDA stream only; all arithmetic runs in libavc_b200.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import torch
 from torch import Tensor, nn
 
 from . import _lib
-from ._lib import AttackArgs, DecoderDesc, EncoderDesc, HeaderArgs, ModelDesc, WeightView
+from ._lib import AttackArgs, AttackVarlenArgs, DecoderDesc, EncoderDesc, HeaderArgs, ModelDesc, WeightView
 
 
 class AvcError(RuntimeError):
@@ -261,6 +261,93 @@ class Engine:
         if want_loss or want_grad:
             return out, {"losses": loss[:int(n_iters)] if loss is not None else None, "grad": grad, "w0": w0}
         return out
+
+    def _packed(self, mels: Sequence[Tensor], name: str) -> Tensor:
+        """[sum T_i, c_in] time-major block of utterances given as [T_i, c_in] mels: a view when they are consecutive
+        contiguous views of one buffer (as AudioEngine.wav2mel_varlen returns them), else one torch.cat."""
+        for i, m in enumerate(mels):
+            if not isinstance(m, Tensor):
+                raise TypeError(f"{name}[{i}] must be a torch.Tensor")
+            if m.device.type != "cuda":
+                raise AvcError(f"{name}[{i}] is on {m.device}: attack_vc_b200 runs on CUDA only (no CPU fallback)")
+            if m.device != self.device:
+                raise AvcError(f"{name}[{i}] is on {m.device} but the engine lives on {self.device}")
+            if m.dtype != torch.float32 or m.dim() != 2 or m.shape[1] != self.c_in:
+                raise ValueError(f"{name}[{i}] must be a float32 [T, {self.c_in}] mel (got {m.dtype} {tuple(m.shape)})")
+        first, rows, consecutive = mels[0], 0, True
+        for m in mels:
+            consecutive = consecutive and m.is_contiguous() and m.untyped_storage().data_ptr() == first.untyped_storage().data_ptr() \
+                and m.data_ptr() == first.data_ptr() + rows * self.c_in * 4
+            rows += int(m.shape[0])
+        if consecutive:
+            return first.as_strided((rows, self.c_in), (self.c_in, 1))
+        return torch.cat([m.contiguous() for m in mels])
+
+    def attack_varlen(self, kind: str, vc_tgt: Sequence[Tensor], adv_tgt: Tensor, eps: float, n_iters: int,
+                      vc_src: Optional[Tensor] = None, w0=None, inv_norm: Optional[float] = None,
+                      want_loss: bool = False, want_grad: bool = False, use_graph: bool = True):
+        """One attack over utterances of different lengths (avc_attack_varlen).  ``vc_tgt`` is a sequence of [T_i, 80]
+        time-major mels; ``adv_tgt`` / ``vc_src`` are [B, 80, T] as in ``attack`` (batch stride 0 allowed).  ``w0`` is a
+        sequence of [T_i, 80] (or one packed [sum T_i, 80] tensor); None draws it as ``Defender.draw_w0`` does, one
+        utterance at a time in input order.  Returns the defended [T_i, 80] mels (views of one packed output), or
+        ``(mels, info)`` when want_loss / want_grad is set: ``info["grad"]`` holds [T_i, 80] views too.  ``inv_norm``
+        defaults as in ``attack``; the loss curve is summed over the batch."""
+        if kind not in ("emb", "e2e", "fb"):
+            raise NotImplementedError(kind)
+        mels = list(vc_tgt)
+        if not mels:
+            raise ValueError("vc_tgt is empty")
+        frames = [int(m.shape[0]) if isinstance(m, Tensor) and m.dim() == 2 else -1 for m in mels]
+        B = len(mels)
+        with torch.cuda.device(self.device):
+            x = self._packed(mels, "vc_tgt")
+            rows = x.shape[0]
+            adv_tgt = self._utt(adv_tgt, "adv_tgt")
+            if kind != "emb":
+                if vc_src is None:
+                    raise ValueError("vc_src is required for e2e and fb attacks")
+                vc_src = self._utt(vc_src, "vc_src")
+            else:
+                vc_src = None
+            if adv_tgt.shape[0] != B or (vc_src is not None and vc_src.shape[0] != B):
+                raise ValueError("batch sizes of vc_src / vc_tgt / adv_tgt differ")
+            if w0 is None:
+                w0 = [torch.zeros_like(m.t().unsqueeze(0)).normal_(0, 1)[0].t() for m in mels]
+            if isinstance(w0, Tensor):
+                if w0.device != self.device or w0.dtype != torch.float32 or w0.dim() != 2 or w0.shape[1] != self.c_in:
+                    raise ValueError(f"a packed w0 must be a float32 [sum T_i, {self.c_in}] tensor on {self.device}")
+                w = w0.contiguous()
+            else:
+                w0 = list(w0)
+                if len(w0) != B:
+                    raise ValueError(f"w0 has {len(w0)} utterances, vc_tgt {B}")
+                w = self._packed(w0, "w0")
+                if [int(t.shape[0]) for t in w0] != frames:
+                    raise ValueError("w0's utterance lengths differ from vc_tgt's")
+            if w.shape[0] != rows:
+                raise ValueError(f"w0 holds {w.shape[0]} frames, vc_tgt {rows} (sum of the utterance lengths)")
+            n_iters = int(n_iters)
+            out = torch.empty((rows, self.c_in), device=self.device, dtype=torch.float32)
+            loss = torch.zeros(max(n_iters, 1), device=self.device, dtype=torch.float32) if want_loss else None
+            grad = torch.zeros((rows, self.c_in), device=self.device, dtype=torch.float32) if want_grad else None
+            fr = (C.c_int32 * B)(*frames)
+            a = AttackVarlenArgs()
+            a.vc_tgt, a.w0, a.adv_out = x.data_ptr(), w.data_ptr(), out.data_ptr()
+            a.grad_out = grad.data_ptr() if grad is not None else None
+            a.frames_host, a.B = fr, B
+            a.adv_tgt, a.adv_stride, a.T_adv = adv_tgt.data_ptr(), _strides3(adv_tgt), adv_tgt.shape[2]
+            if vc_src is not None:
+                a.vc_src, a.src_stride, a.T_src = vc_src.data_ptr(), _strides3(vc_src), vc_src.shape[2]
+            a.loss_out = loss.data_ptr() if loss is not None else None
+            a.eps, a.n_iters = float(eps), n_iters
+            a.inv_norm = float(inv_norm) if inv_norm is not None else 0.0
+            a.use_graph = 1 if use_graph else 0
+            self._check(self._lib.avc_attack_varlen(self._h, {"emb": 0, "e2e": 1, "fb": 2}[kind], C.byref(a), self._stream()))
+        outs = list(out.split(frames))
+        if want_loss or want_grad:
+            return outs, {"losses": loss[:n_iters] if loss is not None else None,
+                          "grad": list(grad.split(frames)) if grad is not None else None, "w0": w}
+        return outs
 
     def begin(self, kind: str, vc_tgt: Tensor, adv_tgt: Tensor, eps: float, n_iters: int,
               vc_src: Optional[Tensor] = None, w0: Optional[Tensor] = None, inv_norm: Optional[float] = None,

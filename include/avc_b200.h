@@ -103,6 +103,31 @@ int avc_e2e_attack(avc_handle* h, const avc_attack_args* a, void* stream);
 /* replaces: attack_utils.fb_attack (attack_utils.py:89-130) */
 int avc_fb_attack(avc_handle* h, const avc_attack_args* a, void* stream);
 
+/* ---- attacks over utterances of DIFFERENT lengths in one call ------------------------------
+ * The same three attacks (kind 0 emb, 1 e2e, 2 fb) on B utterances of frames_host[b] frames each.  The perturbed
+ * utterances only pass through the speaker encoder, which runs them as one padded batch on the tensor-core kernels
+ * with per-utterance lengths; the adversarial target and the conversion source keep one length for the batch.
+ * vc_tgt, w0, adv_out and grad_out are PACKED: utterance b's frames are rows [sum_{i<b} T_i, sum_{i<=b} T_i) of one
+ * contiguous time-major [sum_b T_b, 80] tensor.  loss_out (summed over the batch), eps, n_iters, inv_norm and use_graph
+ * mean what they mean in avc_attack_args.  Every length must pass the speaker encoder's reflect-padding rule; the
+ * error names the first utterance that does not.  AVC_CONV_IMPL=1 or 3 (CUDA cores) is rejected. */
+typedef struct avc_attack_varlen_args {
+  const float* vc_tgt;        /* [sum T_b, 80] packed utterances to defend                        */
+  const float* w0;            /* [sum T_b, 80] packed initial w                                   */
+  float* adv_out;             /* [sum T_b, 80] packed result                                      */
+  float* grad_out;            /* [sum T_b, 80] packed dL/dw of the last iteration; may be NULL    */
+  const int32_t* frames_host; /* [B] host: frames of every utterance                              */
+  int32_t B;
+  const float* adv_tgt; int64_t adv_stride[3]; int32_t T_adv;   /* [B,80,T_adv], batch stride 0 allowed */
+  const float* vc_src;  int64_t src_stride[3]; int32_t T_src;   /* NULL for emb                         */
+  float* loss_out;            /* [n_iters] device or NULL                                         */
+  float eps;
+  int32_t n_iters;
+  double inv_norm;
+  int32_t use_graph;
+} avc_attack_varlen_args;
+int avc_attack_varlen(avc_handle* h, int32_t kind, const avc_attack_varlen_args* a, void* stream);
+
 /* ---- the same attacks as a session, so a caller can interleave iterations with a progress bar
  * (the reference shows tqdm.trange, attack_utils.py:33,71,115) or time iterations precisely.
  * begin: validates, computes targets + loop invariants, captures one iteration (kind 0 emb, 1 e2e,

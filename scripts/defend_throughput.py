@@ -8,6 +8,8 @@ and speaker statistics taken from the synthetic corpus's own mels: one ragged fr
 length, one ragged back-end call.  With ``--gpus N`` one process per GPU defends its own slice and the waveforms are
 all-gathered at the end (NCCL), inside the timed region.  One warm-up defence at the timed shapes, then one timed
 defence: host clock around a call that ends in torch.cuda.synchronize(), CUDA events per stage.  Prints one JSON line.
+``--mixed-lengths`` runs the attacks as ragged calls over chunks of the length-sorted utterances (``defend(...,
+mixed_lengths=True)``) instead of grouping them by length.
 """
 from __future__ import annotations
 
@@ -74,7 +76,8 @@ def run(rank: int, world: int, port: int, args, q):
 
     def once():
         torch.manual_seed(rank)
-        out = d.defend(wavs, adv, attack_type=args.attack, n_iters=args.iters, vc_src=src, griffin_lim_iters=args.gl_iters)
+        out = d.defend(wavs, adv, attack_type=args.attack, n_iters=args.iters, vc_src=src, griffin_lim_iters=args.gl_iters,
+                       mixed_lengths=args.mixed_lengths)
         if world > 1:
             out = gather_varlen(out, B_total, dev)
         torch.cuda.synchronize(dev)
@@ -106,6 +109,7 @@ def main():
     ap.add_argument("--utterances", type=int, default=512, help="utterances per GPU")
     ap.add_argument("--frames", type=int, default=512)
     ap.add_argument("--ragged", action="store_true")
+    ap.add_argument("--mixed-lengths", action="store_true", help="ragged attack calls over length-sorted chunks")
     ap.add_argument("--iters", type=int, default=1500)
     ap.add_argument("--gl-iters", type=int, default=100)
     ap.add_argument("--gpus", type=int, default=1)
@@ -141,7 +145,7 @@ def main():
     total = sum(r["utterances"] for r in ranks)
     print(json.dumps(dict(
         metric="defended utterances/s", attack=args.attack, utterances_per_gpu=args.utterances, frames=args.frames,
-        ragged=args.ragged, iters=args.iters, gl_iters=args.gl_iters, gpus=args.gpus, seconds=round(sec, 4),
+        ragged=args.ragged, mixed_lengths=args.mixed_lengths, iters=args.iters, gl_iters=args.gl_iters, gpus=args.gpus, seconds=round(sec, 4),
         utt_per_s_total=round(total / sec, 3), utt_per_s_per_gpu=round(total / sec / args.gpus, 3),
         stages_ms_rank0={k: round(v, 3) for k, v in ranks[0]["stages_ms"].items()},
         kernel_launches_rank0=ranks[0]["kernel_launches"], gpu=name, power_limit_and_max_sm_clock=limits)))
